@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""bench.py — the hot path's headline measurement (contract: task brief ④).
+"""bench.py — the hot path's headline measurement.
 
 Workload (config.workload): BASELINE.json configs[3], the HBM-streaming case the
 roofline ceilings of BASELINE.md are quoted on — a synthetic batch of 64 noisy
@@ -14,6 +14,10 @@ A "step" is one such pass = 64·512·512·1000 = 16.78 Gpixel-iterations per GPU
            stack inside the timed region.
   --impl reference — the reference algorithm on the box's host cores (the C oracle
            port, OpenMP over images; Julia is not installed anywhere: DESIGN.md).
+  --dump-outputs DIR — what the last timed step handed back (rank 0): DIR/costgrad.npy, the [loss, gradient] pair,
+           and DIR/u_sample.npy, the denoised stack at 2^22 fixed, seeded positions of its column-major M×N×O
+           layout (the whole stack is 128 MiB), both float64.  The inputs are seeded, so two builds run with the same
+           arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -222,7 +226,11 @@ def main():
     ap.add_argument("--impl", default="bpltv", choices=["bpltv", "reference"])
     ap.add_argument("--arith", default="strict", choices=["strict", "fast"])
     ap.add_argument("--no-extras", action="store_true", help="skip the learn_eval wall-time extras")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs as DIR/<name>.npy (costgrad, u_sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -278,10 +286,13 @@ def main():
             # every rank fails or succeeds together (the id broadcast is collective, the NCCL binding is the same file)
             collective = f"torch.distributed all_reduce (library communicator unavailable: {type(e).__name__}: {e})"
 
-    def step():
-        ctx.learn_eval_device(LAM, 0.1, d_costgrad.data_ptr(), eopts, stream=stream)
+    def step(d_u_ptr=0):
+        ctx.learn_eval_device(LAM, 0.1, d_costgrad.data_ptr(), eopts, d_u_ptr=d_u_ptr, stream=stream)
         if world > 1 and not lib_comm:
             dist.all_reduce(d_costgrad)
+
+    # --dump-outputs: the last timed step also hands back the denoised stack (one device-to-device copy of it)
+    d_u = torch.empty((O_PER_GPU, N, M), dtype=torch.float64, device=dev) if args.dump_outputs else None
 
     for _ in range(W):
         step()
@@ -295,8 +306,8 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     with ClockSampler(local) as clk:
         e0.record(tstream)
-        for _ in range(K):
-            step()
+        for k in range(K):
+            step(d_u.data_ptr() if d_u is not None and k == K - 1 else 0)
         e1.record(tstream)
         torch.cuda.synchronize()
     if world > 1:
@@ -311,6 +322,9 @@ def main():
     pix_iter_per_step = float(M) * N * O_PER_GPU * ITERS
     value = pix_iter_per_step * world / (ms_per_step * 1e-3) / 1e9
     loss = float(d_costgrad[0].item())   # after the all-reduce: the loss of the whole job
+    if d_u is not None and rank == 0:
+        dump_outputs(args.dump_outputs, d_costgrad.cpu().numpy(), d_u.cpu().numpy())
+        del d_u
 
     # ---- the same leg in the fast arithmetic mode (FMA, rsqrt; within 1e-10 of the oracle) ----
     value_other = None
@@ -484,6 +498,15 @@ def main():
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+def dump_outputs(out_dir, costgrad, u_onm):
+    """`u_onm`: the denoised stack as the contiguous (O, N, M) array, i.e. the column-major M×N×O layout."""
+    os.makedirs(out_dir, exist_ok=True)
+    u = u_onm.ravel()
+    idx = np.sort(np.random.default_rng(20240601).choice(u.size, size=min(u.size, 1 << 22), replace=False))
+    np.save(os.path.join(out_dir, "costgrad.npy"), np.asarray(costgrad, dtype=np.float64))
+    np.save(os.path.join(out_dir, "u_sample.npy"), u[idx].astype(np.float64))
 
 
 def config5_extra(bp, torch, dist, dev, tstream, world, rank, local, total=1024, n=256, iters=5000):
