@@ -132,6 +132,22 @@ static __device__ __forceinline__ float lds1(tb_addr addr, float)
 }
 #endif
 
+// a > b as a 0/1 word.  Opaque to the front end on purpose: it turns a thread's OR of the ball tests `n² > α²` into
+// a maximum of the n² (an fmax chain with NaN handling, about seven instructions per pixel against two here).
+#ifdef BPLTV_EMU
+template <typename Real>
+static inline unsigned tb_gt(Real a, Real b) { return a > b ? 1u : 0u; }
+#else
+static __device__ __forceinline__ unsigned tb_gt(double a, double b)
+{
+    unsigned r; asm("{\n.reg .pred p;\nsetp.gt.f64 p, %1, %2;\nselp.u32 %0, 1, 0, p;\n}" : "=r"(r) : "d"(a), "d"(b)); return r;
+}
+static __device__ __forceinline__ unsigned tb_gt(float a, float b)
+{
+    unsigned r; asm("{\n.reg .pred p;\nsetp.gt.f32 p, %1, %2;\nselp.u32 %0, 1, 0, p;\n}" : "=r"(r) : "f"(a), "f"(b)); return r;
+}
+#endif
+
 template <typename Real, int T>
 struct TBlockArgs {
     const Real *x_in, *y1_in, *y2_in, *f;
@@ -162,6 +178,8 @@ struct TBSeg {
     bool st_ok;        // this thread owns rows (threads beyond the column compute a copy, store nothing)
     bool multi_warp;
     Real alpha_s;
+    Real alpha2;       // RN(α²) of the scalar α (strict arithmetic): the ball's test, once per segment
+    bool alpha_ok;     // BallScale's α range test of the scalar α
     // column prefetch ring (RING kernels), shared-window byte addresses of this thread's rows:
     // slot i of {x,y1,y2} at ring_t + i·3·colb (planes colb apart), slot j of f at fring_t + j·colb;
     // image column c of the segment is load number k0 + (c - cs)
@@ -169,6 +187,14 @@ struct TBSeg {
     unsigned colb;
     int k0;
 };
+
+template <typename Real>
+static __device__ __forceinline__ void tb_set_alpha(TBSeg<Real> &g, Real al)
+{
+    g.alpha_s = al;
+    g.alpha2 = StrictOps<Real>::mul(al, al);
+    g.alpha_ok = BallScale<Real>::fast_ok_alpha(al);
+}
 
 // thread 0: start the TMA copies of image column `col` (load number kk)
 template <typename Real, int T>
@@ -265,9 +291,13 @@ static __device__ __forceinline__ void tblock_step(const int c, const TBStage<Re
     // ---------------- D-phase ---------------------------------------------------------------
     // Δy1 of the new column; dual ascent v = y + σ∇x̄ of column p-1 for every active stage
     Real v1[T][VEC], v2[T][VEC], n2[T][VEC], al[T][VEC];
-    bool outside = false;
+    unsigned out[T][VEC], outside = 0;      // out: n² > α² (strict arithmetic, scalar α)
+    // scalar α: stages in descending order, so that stage s reads its input duals before stage s-1 forms the ones it
+    // hands on (see the end of the step) and the two never need registers at the same time.  The λ-map kernels keep
+    // the ascending order and the per-pixel α² and select of the projection: on them the scalar form measured slower.
 #pragma unroll
-    for (int s = 0; s < T; ++s) {
+    for (int i = 0; i < T; ++i) {
+        const int s = MAP ? i : T - 1 - i;
         const int p = c - 2 * s;
         if (do_primal[s]) {
             Real dn = __shfl_down_sync(0xffffffffu, xb_c[s][0], 1);
@@ -275,12 +305,12 @@ static __device__ __forceinline__ void tblock_step(const int c, const TBStage<Re
 #pragma unroll
             for (int v = 0; v < VEC; ++v) {
                 const Real nxt = (v == VEC - 1) ? dn : xb_c[s][v + 1];
-                const bool last_row = (r0 + v == M - 1);
+                const bool last_row = v == VEC - 1 && r0 + v == M - 1;   // M % VEC == 0
                 C[s].d1[v] = last_row ? (Real)0 : (STRICT ? A::sub(nxt, xb_c[s][v]) : nxt - xb_c[s][v]);
             }
         }
 #pragma unroll
-        for (int v = 0; v < VEC; ++v) { v1[s][v] = v2[s][v] = n2[s][v] = 0; al[s][v] = g.alpha_s; }
+        for (int v = 0; v < VEC; ++v) { v1[s][v] = v2[s][v] = n2[s][v] = 0; al[s][v] = g.alpha_s; out[s][v] = 0; }
         if (do_dual[s] || do_flush[s]) {
             if (MAP) IO::ld(g.amap + (size_t)(p - 1) * M + r0, al[s]);
 #pragma unroll
@@ -291,7 +321,12 @@ static __device__ __forceinline__ void tblock_step(const int c, const TBStage<Re
                     v1[s][v] = A::add(P[s].y1[v], A::mul(scs[s].sigma, P[s].d1[v]));
                     v2[s][v] = A::add(P[s].y2[v], A::mul(scs[s].sigma, d2));
                     n2[s][v] = A::add(A::mul(v1[s][v], v1[s][v]), A::mul(v2[s][v], v2[s][v]));
-                    outside |= n2[s][v] > A::mul(al[s][v], al[s][v]);
+                    if (MAP) {
+                        outside |= n2[s][v] > A::mul(al[s][v], al[s][v]);
+                    } else {
+                        out[s][v] = tb_gt(n2[s][v], g.alpha2);
+                        outside |= out[s][v];
+                    }
                 } else {
                     if (do_dual[s]) d2 = xb_c[s][v] - P[s].xb[v];
                     v1[s][v] = fma_(scs[s].sigma, P[s].d1[v], P[s].y1[v]);
@@ -306,18 +341,18 @@ static __device__ __forceinline__ void tblock_step(const int c, const TBStage<Re
     // that left the ball are scaled in one block so that their √ and ÷ chains overlap (a
     // thread none of whose pixels left the ball skips it entirely)
     if (outside) {
-        if (STRICT) {
+        if (STRICT && MAP) {
             // α / sqrt(n²) with both operations correctly rounded, as branch-free chains (BallScale, common.cuh): the
             // T·VEC chains of the thread interleave; a pixel outside the chain's operand range (never on image data)
             // sends the thread's pixels through the IEEE operations instead
             Real sc[T][VEC];
-            bool out[T][VEC], ok = true;
+            bool outm[T][VEC], ok = true;
 #pragma unroll
             for (int s = 0; s < T; ++s)
 #pragma unroll
                 for (int v = 0; v < VEC; ++v) {
-                    out[s][v] = n2[s][v] > A::mul(al[s][v], al[s][v]);
-                    if (!out[s][v]) n2[s][v] = (Real)1;
+                    outm[s][v] = n2[s][v] > A::mul(al[s][v], al[s][v]);
+                    if (!outm[s][v]) n2[s][v] = (Real)1;
                     ok &= BallScale<Real>::fast_ok(n2[s][v], al[s][v]);
                 }
 #pragma unroll
@@ -334,7 +369,46 @@ static __device__ __forceinline__ void tblock_step(const int c, const TBStage<Re
             for (int s = 0; s < T; ++s)
 #pragma unroll
                 for (int v = 0; v < VEC; ++v)
-                    if (out[s][v]) { v1[s][v] = A::mul(v1[s][v], sc[s][v]); v2[s][v] = A::mul(v2[s][v], sc[s][v]); }
+                    if (outm[s][v]) { v1[s][v] = A::mul(v1[s][v], sc[s][v]); v2[s][v] = A::mul(v2[s][v], sc[s][v]); }
+        } else if (STRICT) {
+            // α / sqrt(n²) with both operations correctly rounded, as branch-free chains (BallScale, common.cuh): the
+            // T·VEC chains of the thread interleave; a pixel outside the chain's operand range (never on image data)
+            // sends the thread's pixels through the IEEE operations instead.  The scalar α is checked once per segment.
+            //   A pixel inside the ball goes through the chain with n² := α², and its factor RN(α / RN(√RN(α²))) is
+            // exactly 1: RN(√RN(α²)) = α for every α > 0 whose square neither overflows nor underflows in binary
+            // floating point (Boldo, "Stupid is as stupid does: taking the square root of the square of a floating-point
+            // number", 2015), which the α range of fast_ok guarantees.  Multiplying by 1 is exact for every non-NaN
+            // operand (±0, subnormals and ±inf included), so every pixel is scaled without a select of the factor or of
+            // the products.  The IEEE path selects explicitly (its α need not be positive).
+            Real sc[T][VEC];
+            bool ok = g.alpha_ok;
+#pragma unroll
+            for (int s = 0; s < T; ++s)
+#pragma unroll
+                for (int v = 0; v < VEC; ++v) {
+                    if (!out[s][v]) n2[s][v] = g.alpha2;
+                    ok &= BallScale<Real>::fast_ok_a(n2[s][v]);
+                }
+#pragma unroll
+            for (int s = 0; s < T; ++s)
+#pragma unroll
+                for (int v = 0; v < VEC; ++v) sc[s][v] = BallScale<Real>::eval(n2[s][v], al[s][v]);
+            if (!ok) {
+#pragma unroll
+                for (int s = 0; s < T; ++s)
+#pragma unroll
+                    for (int v = 0; v < VEC; ++v) {
+                        const Real q = ball_scale_ieee<Real>(n2[s][v], al[s][v]);
+                        sc[s][v] = n2[s][v] > g.alpha2 ? q : (Real)1;
+                    }
+            }
+#pragma unroll
+            for (int s = 0; s < T; ++s)
+#pragma unroll
+                for (int v = 0; v < VEC; ++v) {
+                    v1[s][v] = A::mul(v1[s][v], sc[s][v]);
+                    v2[s][v] = A::mul(v2[s][v], sc[s][v]);
+                }
         } else {
 #pragma unroll
             for (int s = 0; s < T; ++s)
@@ -398,7 +472,8 @@ __global__ void __launch_bounds__(MAXT, MINB) pdps_tblock_kernel(const TBlockArg
 
     const int M = a.M, N = a.N;
     TBSeg<Real> g;
-    g.M = M; g.N = N; g.amap = a.alpha_map; g.alpha_s = a.alpha_s;
+    g.M = M; g.N = N; g.amap = a.alpha_map;
+    tb_set_alpha(g, a.alpha_s);
     g.st_ok = (int)threadIdx.x * VEC < M;                 // M % VEC == 0 → all VEC rows valid together
     g.r0 = min((int)threadIdx.x * VEC, M - VEC);          // threads beyond the column shadow its last rows
     g.lane = threadIdx.x & 31; g.warp = threadIdx.x >> 5;
@@ -433,7 +508,7 @@ __global__ void __launch_bounds__(MAXT, MINB) pdps_tblock_kernel(const TBlockArg
         if (BATCH) {
             g.fin = a.f + (size_t)a.bm.f_image(o) * M * N;
             if (MAP) g.amap = a.alpha_map + (size_t)a.bm.lam_set(o) * a.bm.map_stride;
-            g.alpha_s = a.bm.scalar(o, a.alpha_s);
+            tb_set_alpha(g, a.bm.scalar(o, a.alpha_s));
         } else {
             g.fin = a.f + img;
         }
