@@ -224,7 +224,8 @@ struct Dev {
     int sm_count = 0;
     size_t smem_optin = 0;
     cudaStream_t stream = nullptr;
-    cudaEvent_t ev[8] = {nullptr};
+    cudaEvent_t ev[8] = {nullptr};   // phase marks of the current call (Mark below)
+    unsigned marked = 0;             // … which of them it has recorded
     // resident dataset shard
     int M = 0, N = 0, O = 0;  // O = images on this device
     int o_begin = 0;          // first global image index of the shard
@@ -235,9 +236,8 @@ struct Dev {
     GradWork grad3;           // gradient_sumregs.cuh
     NdWork *nd = nullptr;     // gradient_nd.cuh (nested-dissection adjoint solver), created on first use
     NdWork *nd3 = nullptr;    // the same solver at coupling radius 2 (scalar sumregs_gradient_reg); a plan of its own
-    bool grad_used_nd = false;
-    bool grad3_used_nd = false;
-    bool grad_used_band = false; // a banded factorisation ran: its worst backward error is in grad.relres_max (device)
+    // the solver of the last gradient on this device: its worst backward error is in its workspace (device memory)
+    enum LastGrad { GRAD_NONE, GRAD_TV_ND, GRAD_TV_BAND, GRAD_SR_ND, GRAD_SR_BAND } last_grad = GRAD_NONE;
     StepKey steps_key;
     std::vector<unsigned char> steps_host;
     long long launches = 0;
@@ -839,6 +839,78 @@ static float ev_ms(cudaEvent_t a, cudaEvent_t b)
     return ms;
 }
 
+// Phase boundaries of one call on one device, recorded as Dev::ev[mark] on the stream the work goes to.  A call marks
+// the boundaries it passes; a phase runs from the previous mark to its own, and a phase that is not marked stays 0 in
+// the stats.  ms_total runs from MARK_BEGIN to MARK_DOWNLOAD.
+enum Mark { MARK_BEGIN, MARK_UPLOAD, MARK_SOLVE, MARK_COST, MARK_GRADIENT, MARK_DOWNLOAD, N_MARKS };
+
+static int mark(Dev &d, Mark m, cudaStream_t st)
+{
+    CU_TRY(cudaEventRecord(d.ev[m], st));
+    d.marked |= 1u << m;
+    return 0;
+}
+
+// kernel launches and phase times (maxima over the devices) of one device's part of a call, after its stream has
+// been synchronised
+static void fold_device_stats(bpltv_stats &s, const Dev &d)
+{
+    double *ms[N_MARKS] = {nullptr, &s.ms_upload, &s.ms_pdps, &s.ms_cost, &s.ms_gradient, &s.ms_download};
+    int prev = -1;
+    for (int m = 0; m < N_MARKS; ++m) {
+        if (!(d.marked >> m & 1)) continue;
+        if (prev >= 0) *ms[m] = std::max<double>(*ms[m], ev_ms(d.ev[prev], d.ev[m]));
+        prev = m;
+    }
+    const unsigned ends = 1u << MARK_BEGIN | 1u << MARK_DOWNLOAD;
+    if ((d.marked & ends) == ends) s.ms_total = std::max<double>(s.ms_total, ev_ms(d.ev[MARK_BEGIN], d.ev[MARK_DOWNLOAD]));
+    s.kernel_launches += d.launches;
+}
+
+// The three passes of a host-pointer entry point over the context's devices, each in device order:
+//  1. enqueue(d, di): the shard's uploads, solve, cost and gradient, the all-reduce and the D2H copy of [cost, grad];
+//  2. download(d, di): the downloads of u.  A pass of their own: a pageable destination makes a download wait for its
+//     device, which must not hold back the other devices' work;
+//  3. fold(d, di), once the device's stream has been synchronised: the host sums (in device order, hence
+//     deterministic) and the stats.
+// skip_empty: devices whose shard of the resident dataset has no images take no part.
+template <class Enqueue, class Download, class Fold>
+static int run_sharded(bpltv_ctx *ctx, bool skip_empty, Enqueue &&enqueue, Download &&download, Fold &&fold)
+{
+    auto each = [&](auto &&pass) {
+        for (int di = 0; di < (int)ctx->devs.size(); ++di) {
+            Dev &d = ctx->devs[di];
+            if (skip_empty && d.O == 0) continue;
+            CU_TRY(cudaSetDevice(d.id));
+            RC_TRY(pass(d, di));
+        }
+        return 0;
+    };
+    RC_TRY(each([&](Dev &d, int di) {
+        d.launches = 0;
+        d.marked = 0;
+        d.last_grad = Dev::GRAD_NONE;
+        return enqueue(d, di);
+    }));
+    RC_TRY(each(download));
+    return each([&](Dev &d, int di) {
+        CU_TRY(cudaStreamSynchronize(d.stream));
+        fold(d, di);
+        return 0;
+    });
+}
+
+static int no_download(Dev &, int) { return 0; }
+
+// second pass of the evaluations: this device's shard of the resident dataset's u (u_out may be NULL)
+template <typename Real>
+static int download_resident_u(Dev &d, const Real *u, double *u_out)
+{
+    const size_t plane = (size_t)d.M * d.N;
+    if (u_out && d.O > 0) RC_TRY(download_stack<Real>(d, u, plane * d.O, u_out + plane * d.o_begin, d.stream));
+    return mark(d, MARK_DOWNLOAD, d.stream);
+}
+
 template <typename Real>
 static int denoise_impl(bpltv_ctx *ctx, const double *noisy, int M, int N, int O, const double *lam, int lm, int ln,
                         const bpltv_pdps_opts &o, double *u_out)
@@ -846,64 +918,41 @@ static int denoise_impl(bpltv_ctx *ctx, const double *noisy, int M, int N, int O
     const int ndev = (int)ctx->devs.size();
     const size_t plane = (size_t)M * N;
     std::memset(&ctx->stats, 0, sizeof ctx->stats);
-    // pass 1: every device gets its shard and its solve enqueued; pass 2: the downloads (a pageable destination makes
-    // download_stack wait for the device, which must not hold back the other devices' work)
     std::vector<const Real *> us(ndev, nullptr);
     std::vector<int> obs(ndev, 0), ocs(ndev, 0);
-    std::vector<char> piped_dev(ndev, 0);      // the solve carried its own copies (PipeIO)
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        d.launches = 0;
-        int ob, oc;
+    std::vector<char> piped(ndev, 0);      // the solve carried its own copies (PipeIO)
+    auto enqueue = [&](Dev &d, int di) {
+        int &ob = obs[di], &oc = ocs[di];
         if (noisy) shard_range(O, ndev, di, ob, oc);
         else { ob = d.o_begin; oc = d.O; }
-        obs[di] = ob; ocs[di] = oc;
         cudaStream_t st = d.stream;
-        CU_TRY(cudaEventRecord(d.ev[0], st));
-        const Real *f;
+        RC_TRY(mark(d, MARK_BEGIN, st));
         PipeIO pio;
-        bool piped = false;
         if (noisy && oc > 0) {
             int k_ = 0, t_ = 1;
             RC_TRY(choose_pdps_kernel<Real>(d, M, N, oc, o, &k_, &t_));
-            piped = pipe_eligible<Real>(d, M, N, oc, o, k_, t_, noisy + plane * ob, u_out + plane * ob, ndev == 1, &pio);
+            piped[di] = pipe_eligible<Real>(d, M, N, oc, o, k_, t_, noisy + plane * ob, u_out + plane * ob, ndev == 1, &pio);
         }
-        piped_dev[di] = piped;
-        if (noisy && piped) {
-            RC_TRY(d.fbuf.ensure(plane * oc * sizeof(Real)));      // filled chunk by chunk under the first passes
+        const Real *f = d.noisy.as<Real>();
+        if (noisy) {
+            if (piped[di]) RC_TRY(d.fbuf.ensure(plane * oc * sizeof(Real)));      // filled chunk by chunk under the first passes
+            else RC_TRY(upload_stack<Real>(d, noisy + plane * ob, plane * oc, d.fbuf, st));
             f = d.fbuf.as<Real>();
-        } else if (noisy) {
-            RC_TRY(upload_stack<Real>(d, noisy + plane * ob, plane * oc, d.fbuf, st));
-            f = d.fbuf.as<Real>();
-        } else {
-            f = d.noisy.as<Real>();
         }
-        CU_TRY(cudaEventRecord(d.ev[1], st));
+        RC_TRY(mark(d, MARK_UPLOAD, st));
         double alpha_s; const Real *amap;
         RC_TRY(prepare_lambda<Real>(d, lam, lm, ln, M, N, st, &alpha_s, &amap));
         int used = 0, depth = 1;
-        RC_TRY(run_pdps<Real>(d, f, M, N, oc, alpha_s, amap, o, st, &us[di], &used, &depth, nullptr, piped ? &pio : nullptr));
+        RC_TRY(run_pdps<Real>(d, f, M, N, oc, alpha_s, amap, o, st, &us[di], &used, &depth, nullptr, piped[di] ? &pio : nullptr));
         ctx->stats.pdps_kernel_used = used;
         ctx->stats.tblock_depth = depth;
-        CU_TRY(cudaEventRecord(d.ev[2], st));
-    }
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        if (ocs[di] > 0 && !piped_dev[di]) RC_TRY(download_stack<Real>(d, us[di], plane * ocs[di], u_out + plane * obs[di], d.stream));
-        CU_TRY(cudaEventRecord(d.ev[3], d.stream));
-    }
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        CU_TRY(cudaStreamSynchronize(d.stream));
-        ctx->stats.ms_upload = std::max<double>(ctx->stats.ms_upload, ev_ms(d.ev[0], d.ev[1]));
-        ctx->stats.ms_pdps = std::max<double>(ctx->stats.ms_pdps, ev_ms(d.ev[1], d.ev[2]));
-        ctx->stats.ms_download = std::max<double>(ctx->stats.ms_download, ev_ms(d.ev[2], d.ev[3]));
-        ctx->stats.ms_total = std::max<double>(ctx->stats.ms_total, ev_ms(d.ev[0], d.ev[3]));
-        ctx->stats.kernel_launches += d.launches;
-    }
+        return mark(d, MARK_SOLVE, st);
+    };
+    auto download = [&](Dev &d, int di) {
+        if (ocs[di] > 0 && !piped[di]) RC_TRY(download_stack<Real>(d, us[di], plane * ocs[di], u_out + plane * obs[di], d.stream));
+        return mark(d, MARK_DOWNLOAD, d.stream);
+    };
+    RC_TRY(run_sharded(ctx, false, enqueue, download, [&](Dev &d, int) { fold_device_stats(ctx->stats, d); }));
     ctx->stats.pdps_iterations = o.maxiter;
     ctx->stats.pixel_iterations = (long long)plane * O * o.maxiter;
     ctx->stats.n_devices = ndev;
@@ -1006,183 +1055,34 @@ static int sumregs_denoise_impl(bpltv_ctx *ctx, const double *noisy, int M, int 
     const int ndev = (int)ctx->devs.size();
     const size_t plane = (size_t)M * N;
     std::memset(&ctx->stats, 0, sizeof ctx->stats);
-    std::vector<const Real *> us(ndev, nullptr);        // two passes, as in denoise_impl
+    std::vector<const Real *> us(ndev, nullptr);
     std::vector<int> obs(ndev, 0), ocs(ndev, 0);
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        d.launches = 0;
-        int ob, oc;
+    auto enqueue = [&](Dev &d, int di) {
+        int &ob = obs[di], &oc = ocs[di];
         if (noisy) shard_range(O, ndev, di, ob, oc);
         else { ob = d.o_begin; oc = d.O; }
-        obs[di] = ob; ocs[di] = oc;
         cudaStream_t st = d.stream;
-        CU_TRY(cudaEventRecord(d.ev[0], st));
-        const Real *f;
+        RC_TRY(mark(d, MARK_BEGIN, st));
+        const Real *f = d.noisy.as<Real>();
         if (noisy) {
             RC_TRY(upload_stack<Real>(d, noisy + plane * ob, plane * oc, d.fbuf, st));
             f = d.fbuf.as<Real>();
-        } else {
-            f = d.noisy.as<Real>();
         }
-        CU_TRY(cudaEventRecord(d.ev[1], st));
+        RC_TRY(mark(d, MARK_UPLOAD, st));
         Real alpha[3]; const Real *amap;
         RC_TRY(prepare_lambda3<Real>(d, lam, lm, ln, M, N, st, alpha, &amap));
         RC_TRY(run_sumregs_pdps<Real>(d, f, M, N, oc, alpha, amap, o, st, &us[di]));
-        CU_TRY(cudaEventRecord(d.ev[2], st));
-    }
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
+        return mark(d, MARK_SOLVE, st);
+    };
+    auto download = [&](Dev &d, int di) {
         if (ocs[di] > 0) RC_TRY(download_stack<Real>(d, us[di], plane * ocs[di], u_out + plane * obs[di], d.stream));
-        CU_TRY(cudaEventRecord(d.ev[3], d.stream));
-    }
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        CU_TRY(cudaStreamSynchronize(d.stream));
-        ctx->stats.ms_upload = std::max<double>(ctx->stats.ms_upload, ev_ms(d.ev[0], d.ev[1]));
-        ctx->stats.ms_pdps = std::max<double>(ctx->stats.ms_pdps, ev_ms(d.ev[1], d.ev[2]));
-        ctx->stats.ms_download = std::max<double>(ctx->stats.ms_download, ev_ms(d.ev[2], d.ev[3]));
-        ctx->stats.ms_total = std::max<double>(ctx->stats.ms_total, ev_ms(d.ev[0], d.ev[3]));
-        ctx->stats.kernel_launches += d.launches;
-    }
+        return mark(d, MARK_DOWNLOAD, d.stream);
+    };
+    RC_TRY(run_sharded(ctx, false, enqueue, download, [&](Dev &d, int) { fold_device_stats(ctx->stats, d); }));
     ctx->stats.pdps_iterations = o.maxiter;
     ctx->stats.pixel_iterations = (long long)plane * O * o.maxiter;
     ctx->stats.n_devices = ndev;
     ctx->stats.tblock_depth = 1;
-    return 0;
-}
-
-// one sum-of-regularisers evaluation on one device: u, scalars[0] = cost, scalars[1..3·ng] = gradient
-template <typename Real>
-static int sumregs_eval_on_device(bpltv_ctx *ctx, Dev &d, const double *lam, int lm, int ln, double Delta,
-                                  const bpltv_eval_opts &eo, const Real *u_given, cudaStream_t st, const Real **u_res,
-                                  double *d_costgrad)
-{
-    const int M = d.M, N = d.N, O = d.O;
-    const size_t n = (size_t)M * N * O;
-    const int ng = lm * ln;
-    CU_TRY(cudaEventRecord(d.ev[0], st));
-    Real alpha[3]; const Real *amap;
-    RC_TRY(prepare_lambda3<Real>(d, lam, lm, ln, M, N, st, alpha, &amap));
-    const Real *u = u_given;
-    if (!u) RC_TRY(run_sumregs_pdps<Real>(d, d.noisy.as<Real>(), M, N, O, alpha, amap, eo.pdps, st, &u));
-    CU_TRY(cudaEventRecord(d.ev[1], st));
-    CU_TRY(cudaMemsetAsync(d_costgrad, 0, (1 + 3 * ng) * sizeof(double), st));
-    if (O > 0) RC_TRY(run_cost<Real>(d, u, d.truth.as<Real>(), n, d_costgrad, st));
-    CU_TRY(cudaEventRecord(d.ev[2], st));
-    if (O > 0 && eo.force_branch != 3) {
-        Grad3Problem<Real> gp;
-        gp.u = u; gp.ubar = d.truth.as<Real>(); gp.M = M; gp.N = N; gp.O = O;
-        for (int k = 0; k < 3; ++k) gp.alpha[k] = ng == 1 ? lam[k] : 0.0;
-        gp.alpha_maps = amap; gp.lm = lm; gp.ln = ln;
-        gp.regularised = eo.force_branch == 2 || (eo.force_branch == 0 && !(Delta > eo.delta_t));
-        gp.gamma = (gp.regularised && amap && eo.gamma_patch > 0) ? eo.gamma_patch : eo.gamma;   // :200 vs :117
-        gp.act_tol = eo.act_tol;
-        gp.eps_act = eo.eps_act > 0 ? eo.eps_act : 2.220446049250313e-16;   // eps() in both variants (:318-320, :387-389)
-        // scalar sumregs_gradient_reg (:112-167) is symmetric positive definite in node space with coupling radius 2:
-        // nested-dissection multifrontal Cholesky (eval_opts.solver 0 / 2, BPLTV_GRAD_SOLVER); solver 1 or a shape the
-        // fronts do not take: the node-space band LU / compliance form of run_gradient3
-        int solver = eo.solver;
-        if (solver == 0) solver = env_int("BPLTV_GRAD_SOLVER", 0);
-        d.grad3_used_nd = false;
-        int rc = -1;
-        if (gp.regularised && !amap && solver != 1 && M == N) {
-            if (!d.nd3) d.nd3 = nd_work_create();
-            Nd3Problem np;
-            np.u = u; np.ubar = d.truth.as<Real>(); np.prec = (int)sizeof(Real) * 8; np.M = M; np.N = N; np.O = O;
-            for (int k = 0; k < 3; ++k) np.alpha[k] = lam[k];
-            np.gamma = gp.gamma; np.tol = 0.0; np.maxit = eo.solver_maxit;
-            rc = nd_run_gradient3_reg(d.nd3, np, d.sm_count, d.smem_optin, st, d_costgrad + 1, &d.launches);
-            if (rc == 0) d.grad3_used_nd = true;
-            else if (rc == BPLTV_ERR_ALLOC) rc = -1;      // the band solver needs less memory per image
-            else if (rc != -1) return fail(rc, "sumregs gradient: %s", nd_work_error(d.nd3));
-        }
-        // sumregs_gradient (non-regularised, scalar :264-327 and patch :330-407): the same solver in multiplier space
-        // (3-6 unknowns per pixel); fronts beyond shared memory (-1) go to the band Cholesky
-        if (!gp.regularised && solver != 1 && M == N) {
-            if (!d.nd3) d.nd3 = nd_work_create();
-            Nd3mProblem np;
-            np.u = u; np.ubar = d.truth.as<Real>(); np.alpha_maps = amap; np.prec = (int)sizeof(Real) * 8;
-            np.M = M; np.N = N; np.O = O; np.lm = lm; np.ln = ln;
-            for (int k = 0; k < 3; ++k) np.alpha[k] = gp.alpha[k];
-            np.act_tol = gp.act_tol; np.eps_act = gp.eps_act; np.tol = 0.0; np.maxit = eo.solver_maxit;
-            rc = nd_run_gradient3(d.nd3, np, d.sm_count, d.smem_optin, st, d_costgrad + 1, &d.launches);
-            if (rc == 0) d.grad3_used_nd = true;
-            else if (rc == BPLTV_ERR_ALLOC) rc = -1;      // the band Cholesky needs less memory per image
-            else if (rc != -1) return fail(rc, "sumregs gradient: %s", nd_work_error(d.nd3));
-        }
-        if (rc == -1) rc = run_gradient3<Real>(d.grad3, gp, d.sm_count, d.smem_optin, st, d_costgrad + 1, &d.launches);
-        if (rc != 0) return fail(rc == -1 ? BPLTV_ERR_ARG : rc, "sumregs gradient: %s", d.grad3.err.c_str());
-    }
-    CU_TRY(cudaEventRecord(d.ev[3], st));
-    *u_res = u;
-    return 0;
-}
-
-// u_host != NULL: gradient of the caller's u (no solve); else the full learning function
-template <typename Real>
-static int sumregs_learn_eval_impl(bpltv_ctx *ctx, const double *lam, int lm, int ln, double Delta,
-                                   const bpltv_eval_opts &eo, const double *u_host, double *u_out, double *cost_out,
-                                   double *grad_out)
-{
-    const int ndev = (int)ctx->devs.size();
-    const int ng = 3 * lm * ln;
-    const size_t plane = (size_t)ctx->M * ctx->N;
-    std::memset(&ctx->stats, 0, sizeof ctx->stats);
-    std::vector<std::vector<double>> host(ndev, std::vector<double>(1 + ng, 0.0));
-    std::vector<const Real *> us(ndev, nullptr);
-    std::vector<double> relres(ndev, 0.0);
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        d.launches = 0;
-        RC_TRY(d.scalars.ensure((1 + ng) * sizeof(double)));
-        const Real *ug = nullptr;
-        if (u_host) {
-            RC_TRY(upload_stack<Real>(d, u_host + plane * d.o_begin, plane * d.O, d.ubuf, d.stream));
-            ug = d.ubuf.as<Real>();
-        }
-        RC_TRY(sumregs_eval_on_device<Real>(ctx, d, lam, lm, ln, Delta, eo, ug, d.stream, &us[di], d.scalars.as<double>()));
-        RC_TRY(allreduce_costgrad(ctx, d.scalars.as<double>(), 1 + ng, d.stream));
-        CU_TRY(cudaMemcpyAsync(host[di].data(), d.scalars.p, (1 + ng) * sizeof(double), cudaMemcpyDeviceToHost, d.stream));
-        // worst backward error of the banded adjoint solves (grad_reduce_kernel leaves it in the workspace)
-        const void *rr = d.grad3_used_nd ? (const void *)nd_work_relres_max(d.nd3) : (const void *)d.grad3.relres_max;
-        if (d.O > 0 && eo.force_branch != 3 && rr)
-            CU_TRY(cudaMemcpyAsync(&relres[di], rr, sizeof(double), cudaMemcpyDeviceToHost, d.stream));
-    }
-    for (int di = 0; di < ndev; ++di) {      // second pass: see denoise_impl
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        if (u_out && d.O > 0) RC_TRY(download_stack<Real>(d, us[di], plane * d.O, u_out + plane * d.o_begin, d.stream));
-        CU_TRY(cudaEventRecord(d.ev[4], d.stream));
-    }
-    double cost = 0.0;
-    std::vector<double> grad(ng, 0.0);
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        CU_TRY(cudaStreamSynchronize(d.stream));
-        cost += host[di][0];
-        ctx->stats.solver_max_relres = std::max(ctx->stats.solver_max_relres, relres[di]);
-        for (int k = 0; k < ng; ++k) grad[k] += host[di][1 + k];
-        ctx->stats.ms_pdps = std::max<double>(ctx->stats.ms_pdps, ev_ms(d.ev[0], d.ev[1]));
-        ctx->stats.ms_cost = std::max<double>(ctx->stats.ms_cost, ev_ms(d.ev[1], d.ev[2]));
-        ctx->stats.ms_gradient = std::max<double>(ctx->stats.ms_gradient, ev_ms(d.ev[2], d.ev[3]));
-        ctx->stats.ms_download = std::max<double>(ctx->stats.ms_download, ev_ms(d.ev[3], d.ev[4]));
-        ctx->stats.ms_total = std::max<double>(ctx->stats.ms_total, ev_ms(d.ev[0], d.ev[4]));
-        ctx->stats.kernel_launches += d.launches;
-    }
-    ctx->stats.pdps_iterations = u_host ? 0 : eo.pdps.maxiter;
-    ctx->stats.pixel_iterations = u_host ? 0 : (long long)plane * ctx->O * eo.pdps.maxiter;
-    ctx->stats.n_devices = ndev;
-    ctx->stats.tblock_depth = 1;
-    if (!std::isfinite(cost)) return fail(BPLTV_ERR_NUMERIC, "non-finite cost");
-    for (int k = 0; k < ng; ++k)
-        if (!std::isfinite(grad[k])) return fail(BPLTV_ERR_NUMERIC, "non-finite gradient entry %d", k);
-    if (cost_out) *cost_out = cost;
-    for (int k = 0; k < ng; ++k) grad_out[k] = grad[k];
     return 0;
 }
 
@@ -1191,26 +1091,21 @@ static int set_dataset_impl(bpltv_ctx *ctx, const double *truth, const double *n
 {
     const int ndev = (int)ctx->devs.size();
     const size_t plane = (size_t)M * N;
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
+    auto enqueue = [&](Dev &d, int di) {
         int ob, oc;
         shard_range(O, ndev, di, ob, oc);
         d.M = M; d.N = N; d.O = oc; d.o_begin = ob;
         RC_TRY(upload_stack<Real>(d, truth + plane * ob, plane * oc, d.truth, d.stream));
-        RC_TRY(upload_stack<Real>(d, noisy + plane * ob, plane * oc, d.noisy, d.stream));
-    }
-    for (int di = 0; di < ndev; ++di) {
-        CU_TRY(cudaSetDevice(ctx->devs[di].id));
-        CU_TRY(cudaStreamSynchronize(ctx->devs[di].stream));
-    }
+        return upload_stack<Real>(d, noisy + plane * ob, plane * oc, d.noisy, d.stream);
+    };
+    RC_TRY(run_sharded(ctx, false, enqueue, no_download, [](Dev &, int) {}));
     ctx->M = M; ctx->N = N; ctx->O = O; ctx->have_dataset = true;
     return 0;
 }
 
-// Enqueue one evaluation on one device: u = denoise; scalars[0] = cost;
-// scalars[1..] = gradient.  Everything asynchronous on `st`.
-
+// ---------------------------------------------------------------------------
+// gradients: which solver takes the adjoint systems
+// ---------------------------------------------------------------------------
 // gradient / gradient_reg of the TV learning function.  The regularised branch has two implementations:
 // the multiplier-space banded Cholesky of gradient.cuh and the node-space band LU of lu_band.cuh
 // (n² unknowns with half-bandwidth n instead of ≤ 2n² modes with half-bandwidth ≤ 2n+1; its cost does not grow
@@ -1228,8 +1123,7 @@ static int run_tv_gradient(Dev &d, const GradProblem<Real> &gp, cudaStream_t st,
 {
     int solver = gp.solver;
     if (solver == 0) solver = env_int("BPLTV_GRAD_SOLVER", 0);
-    d.grad_used_nd = false;
-    d.grad_used_band = false;
+    d.last_grad = Dev::GRAD_NONE;
     if (solver != 1) {
         if (!d.nd) d.nd = nd_work_create();
         NdProblem np;
@@ -1237,7 +1131,7 @@ static int run_tv_gradient(Dev &d, const GradProblem<Real> &gp, cudaStream_t st,
         np.alpha_s = gp.alpha_s; np.alpha_map = gp.alpha_map; np.lm = gp.lm; np.ln = gp.ln; np.regularised = gp.regularised;
         np.gamma = gp.gamma; np.act_tol = gp.act_tol; np.eps_act = gp.eps_act; np.tol = gp.tol; np.maxit = gp.maxit;
         const int rc = nd_run_gradient(d.nd, np, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
-        if (rc == 0) { d.grad_used_nd = true; return 0; }
+        if (rc == 0) { d.last_grad = Dev::GRAD_TV_ND; return 0; }
         if (rc != -1) { d.grad.err = nd_work_error(d.nd); return rc; }
         // -1: fronts beyond shared memory for this image size — the band solver takes over
     }
@@ -1249,22 +1143,93 @@ static int run_tv_gradient(Dev &d, const GradProblem<Real> &gp, cudaStream_t st,
         lp.alpha[0] = gp.alpha_s; lp.alpha[1] = lp.alpha[2] = 0.0;
         lp.alpha_maps = gp.alpha_map; lp.lm = gp.lm; lp.ln = gp.ln; lp.gamma = gp.gamma; lp.nops = 1;
         const int rc = run_gradient_lu<Real>(d.grad, lp, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
-        if (rc == 0) d.grad_used_band = true;
+        if (rc == 0) d.last_grad = Dev::GRAD_TV_BAND;
         if (rc != -1) return rc;      // -1: the LU does not take this shape (panels beyond shared memory): Cholesky
     }
     const int rc = run_gradient<Real>(d.grad, gp, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
-    if (rc == 0) d.grad_used_band = true;
+    if (rc == 0) d.last_grad = Dev::GRAD_TV_BAND;
+    return rc;
+}
+
+// The sum-of-regularisers gradient (eval_opts.solver as above).  Scalar sumregs_gradient_reg (:112-167) is symmetric
+// positive definite in node space with coupling radius 2, and sumregs_gradient (non-regularised, scalar :264-327 and
+// patch :330-407) is the same in multiplier space (3-6 unknowns per pixel): both take the nested-dissection
+// multifrontal Cholesky.  Solver 1, the patch sumregs_gradient_reg, a shape the fronts do not take (-1) or one that
+// does not fit in memory go to the node-space band LU / compliance-form band Cholesky of run_gradient3, which needs
+// less memory per image.
+template <typename Real>
+static int run_sumregs_gradient(Dev &d, const Grad3Problem<Real> &gp, int solver, int maxit, cudaStream_t st,
+                                double *d_grad_out)
+{
+    if (solver == 0) solver = env_int("BPLTV_GRAD_SOLVER", 0);
+    d.last_grad = Dev::GRAD_NONE;
+    if (solver != 1 && gp.M == gp.N && !(gp.regularised && gp.alpha_maps)) {
+        if (!d.nd3) d.nd3 = nd_work_create();
+        int rc;
+        if (gp.regularised) {
+            Nd3Problem np;
+            np.u = gp.u; np.ubar = gp.ubar; np.prec = (int)sizeof(Real) * 8; np.M = gp.M; np.N = gp.N; np.O = gp.O;
+            for (int k = 0; k < 3; ++k) np.alpha[k] = gp.alpha[k];
+            np.gamma = gp.gamma; np.tol = 0.0; np.maxit = maxit;
+            rc = nd_run_gradient3_reg(d.nd3, np, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
+        } else {
+            Nd3mProblem np;
+            np.u = gp.u; np.ubar = gp.ubar; np.alpha_maps = gp.alpha_maps; np.prec = (int)sizeof(Real) * 8;
+            np.M = gp.M; np.N = gp.N; np.O = gp.O; np.lm = gp.lm; np.ln = gp.ln;
+            for (int k = 0; k < 3; ++k) np.alpha[k] = gp.alpha[k];
+            np.act_tol = gp.act_tol; np.eps_act = gp.eps_act; np.tol = 0.0; np.maxit = maxit;
+            rc = nd_run_gradient3(d.nd3, np, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
+        }
+        if (rc == 0) { d.last_grad = Dev::GRAD_SR_ND; return 0; }
+        if (rc != -1 && rc != BPLTV_ERR_ALLOC) { d.grad3.err = nd_work_error(d.nd3); return rc; }
+    }
+    const int rc = run_gradient3<Real>(d.grad3, gp, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
+    if (rc == 0) d.last_grad = Dev::GRAD_SR_BAND;
     return rc;
 }
 
 // worst backward error of the adjoint solves of the last gradient on this device (device pointer) or nullptr
 static const double *relres_of_last_gradient(const Dev &d)
 {
-    if (d.grad_used_nd) return nd_work_relres_max(d.nd);
-    if (d.grad_used_band) return static_cast<const double *>(d.grad.relres_max);
-    return nullptr;
+    switch (d.last_grad) {
+    case Dev::GRAD_TV_ND: return nd_work_relres_max(d.nd);
+    case Dev::GRAD_TV_BAND: return static_cast<const double *>(d.grad.relres_max);
+    case Dev::GRAD_SR_ND: return nd_work_relres_max(d.nd3);
+    case Dev::GRAD_SR_BAND: return static_cast<const double *>(d.grad3.relres_max);
+    default: return nullptr;
+    }
 }
 
+// end of an evaluation's first pass: [cost, grad] (`count` doubles in d.scalars) summed over the ranks of the job and
+// copied to `host`, with the worst backward error of the device's gradient
+static int fetch_costgrad(bpltv_ctx *ctx, Dev &d, int count, double *host, double *relres)
+{
+    RC_TRY(allreduce_costgrad(ctx, d.scalars.as<double>(), count, d.stream));
+    CU_TRY(cudaMemcpyAsync(host, d.scalars.p, count * sizeof(double), cudaMemcpyDeviceToHost, d.stream));
+    if (relres_of_last_gradient(d))
+        CU_TRY(cudaMemcpyAsync(relres, relres_of_last_gradient(d), sizeof(double), cudaMemcpyDeviceToHost, d.stream));
+    return 0;
+}
+
+// the TV gradient of u against the device's resident truth
+template <typename Real>
+static GradProblem<Real> tv_grad_problem(const Dev &d, const Real *u, double alpha_s, const Real *amap, int lm, int ln,
+                                         bool regularised, const bpltv_eval_opts &eo)
+{
+    GradProblem<Real> gp;
+    gp.u = u; gp.ubar = d.truth.as<Real>(); gp.M = d.M; gp.N = d.N; gp.O = d.O;
+    gp.alpha_s = alpha_s; gp.alpha_map = amap; gp.lm = lm; gp.ln = ln; gp.regularised = regularised;
+    gp.gamma = eo.gamma; gp.act_tol = eo.act_tol;
+    gp.eps_act = eo.eps_act > 0 ? eo.eps_act : (lm * ln == 1 ? 2.220446049250313e-16 : 1.4901161193847656e-08);
+    gp.tol = eo.solver_tol; gp.maxit = eo.solver_maxit; gp.solver = eo.solver;
+    return gp;
+}
+
+// ---------------------------------------------------------------------------
+// evaluations of the learning functions on the resident dataset
+// ---------------------------------------------------------------------------
+// Enqueue one evaluation on one device: u = denoise; scalars[0] = cost;
+// scalars[1..] = gradient.  Everything asynchronous on `st`.
 template <typename Real>
 static int eval_on_device(bpltv_ctx *ctx, Dev &d, const double *lam, int lm, int ln, double Delta,
                           const bpltv_eval_opts &eo, cudaStream_t st, const Real **u_res, double *d_costgrad)
@@ -1272,29 +1237,23 @@ static int eval_on_device(bpltv_ctx *ctx, Dev &d, const double *lam, int lm, int
     const int M = d.M, N = d.N, O = d.O;
     const size_t n = (size_t)M * N * O;
     const int ng = lm * ln;
-    CU_TRY(cudaEventRecord(d.ev[0], st));
+    RC_TRY(mark(d, MARK_BEGIN, st));
     double alpha_s; const Real *amap;
     RC_TRY(prepare_lambda<Real>(d, lam, lm, ln, M, N, st, &alpha_s, &amap));
     const Real *u = nullptr; int used = 0, depth = 1;
     RC_TRY(run_pdps<Real>(d, d.noisy.as<Real>(), M, N, O, alpha_s, amap, eo.pdps, st, &u, &used, &depth));
     ctx->stats.pdps_kernel_used = used;
     ctx->stats.tblock_depth = depth;
-    CU_TRY(cudaEventRecord(d.ev[1], st));
+    RC_TRY(mark(d, MARK_SOLVE, st));
     CU_TRY(cudaMemsetAsync(d_costgrad, 0, (1 + ng) * sizeof(double), st));
     if (O > 0) RC_TRY(run_cost<Real>(d, u, d.truth.as<Real>(), n, d_costgrad, st));
-    CU_TRY(cudaEventRecord(d.ev[2], st));
+    RC_TRY(mark(d, MARK_COST, st));
     if (O > 0 && eo.force_branch != 3) {
         const bool reg = eo.force_branch == 2 || (eo.force_branch == 0 && !(Delta > eo.delta_t));
-        GradProblem<Real> gp;
-        gp.u = u; gp.ubar = d.truth.as<Real>(); gp.M = M; gp.N = N; gp.O = O;
-        gp.alpha_s = alpha_s; gp.alpha_map = amap; gp.lm = lm; gp.ln = ln; gp.regularised = reg;
-        gp.gamma = eo.gamma; gp.act_tol = eo.act_tol;
-        gp.eps_act = eo.eps_act > 0 ? eo.eps_act : (ng == 1 ? 2.220446049250313e-16 : 1.4901161193847656e-08);
-        gp.tol = eo.solver_tol; gp.maxit = eo.solver_maxit; gp.solver = eo.solver;
-        int rc = run_tv_gradient<Real>(d, gp, st, d_costgrad + 1);
+        const int rc = run_tv_gradient<Real>(d, tv_grad_problem<Real>(d, u, alpha_s, amap, lm, ln, reg, eo), st, d_costgrad + 1);
         if (rc != 0) return fail(rc, "gradient: %s", d.grad.err.c_str());
     }
-    CU_TRY(cudaEventRecord(d.ev[3], st));
+    RC_TRY(mark(d, MARK_GRADIENT, st));
     *u_res = u;
     return 0;
 }
@@ -1310,42 +1269,21 @@ static int learn_eval_impl(bpltv_ctx *ctx, const double *lam, int lm, int ln, do
     std::vector<std::vector<double>> host(ndev, std::vector<double>(1 + ng, 0.0));
     std::vector<double> relres(ndev, 0.0);
     std::vector<const Real *> us(ndev, nullptr);
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        d.launches = 0;
-        d.grad_used_nd = d.grad_used_band = false;
-        RC_TRY(d.scalars.ensure((1 + ng) * sizeof(double)));
-        RC_TRY(eval_on_device<Real>(ctx, d, lam, lm, ln, Delta, eo, d.stream, &us[di], d.scalars.as<double>()));
-        RC_TRY(allreduce_costgrad(ctx, d.scalars.as<double>(), 1 + ng, d.stream));
-        CU_TRY(cudaMemcpyAsync(host[di].data(), d.scalars.p, (1 + ng) * sizeof(double), cudaMemcpyDeviceToHost,
-                               d.stream));
-        if (relres_of_last_gradient(d))
-            CU_TRY(cudaMemcpyAsync(&relres[di], relres_of_last_gradient(d), sizeof(double), cudaMemcpyDeviceToHost, d.stream));
-    }
-    for (int di = 0; di < ndev; ++di) {      // second pass: see denoise_impl
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        if (u_out && d.O > 0) RC_TRY(download_stack<Real>(d, us[di], plane * d.O, u_out + plane * d.o_begin, d.stream));
-        CU_TRY(cudaEventRecord(d.ev[4], d.stream));
-    }
     double cost = 0.0;
     std::vector<double> grad(ng, 0.0);
-    for (int di = 0; di < ndev; ++di) {  // fixed device order: deterministic sum
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        CU_TRY(cudaStreamSynchronize(d.stream));
+    auto enqueue = [&](Dev &d, int di) {
+        RC_TRY(d.scalars.ensure((1 + ng) * sizeof(double)));
+        RC_TRY(eval_on_device<Real>(ctx, d, lam, lm, ln, Delta, eo, d.stream, &us[di], d.scalars.as<double>()));
+        return fetch_costgrad(ctx, d, 1 + ng, host[di].data(), &relres[di]);
+    };
+    auto fold = [&](Dev &d, int di) {
         cost += host[di][0];
         for (int k = 0; k < ng; ++k) grad[k] += host[di][1 + k];
-        ctx->stats.ms_pdps = std::max<double>(ctx->stats.ms_pdps, ev_ms(d.ev[0], d.ev[1]));
-        ctx->stats.ms_cost = std::max<double>(ctx->stats.ms_cost, ev_ms(d.ev[1], d.ev[2]));
-        ctx->stats.ms_gradient = std::max<double>(ctx->stats.ms_gradient, ev_ms(d.ev[2], d.ev[3]));
-        ctx->stats.ms_download = std::max<double>(ctx->stats.ms_download, ev_ms(d.ev[3], d.ev[4]));
-        ctx->stats.ms_total = std::max<double>(ctx->stats.ms_total, ev_ms(d.ev[0], d.ev[4]));
-        ctx->stats.kernel_launches += d.launches;
+        fold_device_stats(ctx->stats, d);
         ctx->stats.solver_iterations += d.grad.last_iterations;
         ctx->stats.solver_max_relres = std::max(ctx->stats.solver_max_relres, relres[di]);
-    }
+    };
+    RC_TRY(run_sharded(ctx, false, enqueue, [&](Dev &d, int di) { return download_resident_u<Real>(d, us[di], u_out); }, fold));
     ctx->stats.pdps_iterations = eo.pdps.maxiter;
     ctx->stats.pixel_iterations = (long long)plane * ctx->O * eo.pdps.maxiter;
     ctx->stats.n_devices = ndev;
@@ -1355,6 +1293,86 @@ static int learn_eval_impl(bpltv_ctx *ctx, const double *lam, int lm, int ln, do
             return fail(BPLTV_ERR_NUMERIC, "non-finite gradient entry %d (adjoint solve: worst backward error %.3g, tolerance %.3g)", k,
                         ctx->stats.solver_max_relres, eo.solver_tol);
     *cost_out = cost;
+    for (int k = 0; k < ng; ++k) grad_out[k] = grad[k];
+    return 0;
+}
+
+// one sum-of-regularisers evaluation on one device: u, scalars[0] = cost, scalars[1..3·ng] = gradient
+template <typename Real>
+static int sumregs_eval_on_device(bpltv_ctx *ctx, Dev &d, const double *lam, int lm, int ln, double Delta,
+                                  const bpltv_eval_opts &eo, const Real *u_given, cudaStream_t st, const Real **u_res,
+                                  double *d_costgrad)
+{
+    const int M = d.M, N = d.N, O = d.O;
+    const size_t n = (size_t)M * N * O;
+    const int ng = lm * ln;
+    RC_TRY(mark(d, MARK_BEGIN, st));
+    Real alpha[3]; const Real *amap;
+    RC_TRY(prepare_lambda3<Real>(d, lam, lm, ln, M, N, st, alpha, &amap));
+    const Real *u = u_given;
+    if (!u) RC_TRY(run_sumregs_pdps<Real>(d, d.noisy.as<Real>(), M, N, O, alpha, amap, eo.pdps, st, &u));
+    RC_TRY(mark(d, MARK_SOLVE, st));
+    CU_TRY(cudaMemsetAsync(d_costgrad, 0, (1 + 3 * ng) * sizeof(double), st));
+    if (O > 0) RC_TRY(run_cost<Real>(d, u, d.truth.as<Real>(), n, d_costgrad, st));
+    RC_TRY(mark(d, MARK_COST, st));
+    if (O > 0 && eo.force_branch != 3) {
+        Grad3Problem<Real> gp;
+        gp.u = u; gp.ubar = d.truth.as<Real>(); gp.M = M; gp.N = N; gp.O = O;
+        for (int k = 0; k < 3; ++k) gp.alpha[k] = ng == 1 ? lam[k] : 0.0;
+        gp.alpha_maps = amap; gp.lm = lm; gp.ln = ln;
+        gp.regularised = eo.force_branch == 2 || (eo.force_branch == 0 && !(Delta > eo.delta_t));
+        gp.gamma = (gp.regularised && amap && eo.gamma_patch > 0) ? eo.gamma_patch : eo.gamma;   // :200 vs :117
+        gp.act_tol = eo.act_tol;
+        gp.eps_act = eo.eps_act > 0 ? eo.eps_act : 2.220446049250313e-16;   // eps() in both variants (:318-320, :387-389)
+        const int rc = run_sumregs_gradient<Real>(d, gp, eo.solver, eo.solver_maxit, st, d_costgrad + 1);
+        if (rc != 0) return fail(rc == -1 ? BPLTV_ERR_ARG : rc, "sumregs gradient: %s", d.grad3.err.c_str());
+    }
+    RC_TRY(mark(d, MARK_GRADIENT, st));
+    *u_res = u;
+    return 0;
+}
+
+// u_host != NULL: gradient of the caller's u (no solve; its upload lies outside the timed phases); else the full
+// learning function
+template <typename Real>
+static int sumregs_learn_eval_impl(bpltv_ctx *ctx, const double *lam, int lm, int ln, double Delta,
+                                   const bpltv_eval_opts &eo, const double *u_host, double *u_out, double *cost_out,
+                                   double *grad_out)
+{
+    const int ndev = (int)ctx->devs.size();
+    const int ng = 3 * lm * ln;
+    const size_t plane = (size_t)ctx->M * ctx->N;
+    std::memset(&ctx->stats, 0, sizeof ctx->stats);
+    std::vector<std::vector<double>> host(ndev, std::vector<double>(1 + ng, 0.0));
+    std::vector<const Real *> us(ndev, nullptr);
+    std::vector<double> relres(ndev, 0.0);
+    double cost = 0.0;
+    std::vector<double> grad(ng, 0.0);
+    auto enqueue = [&](Dev &d, int di) {
+        RC_TRY(d.scalars.ensure((1 + ng) * sizeof(double)));
+        const Real *ug = nullptr;
+        if (u_host) {
+            RC_TRY(upload_stack<Real>(d, u_host + plane * d.o_begin, plane * d.O, d.ubuf, d.stream));
+            ug = d.ubuf.as<Real>();
+        }
+        RC_TRY(sumregs_eval_on_device<Real>(ctx, d, lam, lm, ln, Delta, eo, ug, d.stream, &us[di], d.scalars.as<double>()));
+        return fetch_costgrad(ctx, d, 1 + ng, host[di].data(), &relres[di]);
+    };
+    auto fold = [&](Dev &d, int di) {
+        cost += host[di][0];
+        ctx->stats.solver_max_relres = std::max(ctx->stats.solver_max_relres, relres[di]);
+        for (int k = 0; k < ng; ++k) grad[k] += host[di][1 + k];
+        fold_device_stats(ctx->stats, d);
+    };
+    RC_TRY(run_sharded(ctx, false, enqueue, [&](Dev &d, int di) { return download_resident_u<Real>(d, us[di], u_out); }, fold));
+    ctx->stats.pdps_iterations = u_host ? 0 : eo.pdps.maxiter;
+    ctx->stats.pixel_iterations = u_host ? 0 : (long long)plane * ctx->O * eo.pdps.maxiter;
+    ctx->stats.n_devices = ndev;
+    ctx->stats.tblock_depth = 1;
+    if (!std::isfinite(cost)) return fail(BPLTV_ERR_NUMERIC, "non-finite cost");
+    for (int k = 0; k < ng; ++k)
+        if (!std::isfinite(grad[k])) return fail(BPLTV_ERR_NUMERIC, "non-finite gradient entry %d", k);
+    if (cost_out) *cost_out = cost;
     for (int k = 0; k < ng; ++k) grad_out[k] = grad[k];
     return 0;
 }
@@ -1371,15 +1389,13 @@ static int sweep_impl(bpltv_ctx *ctx, const double *lams, int L, int lm, int ln,
     const bool scalar = ng == 1;
     std::memset(&ctx->stats, 0, sizeof ctx->stats);
     std::vector<std::vector<double>> host(ndev);
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        d.launches = 0;
+    std::vector<const Real *> us(ndev, nullptr);
+    std::vector<double> cost(L, 0.0);
+    auto enqueue = [&](Dev &d, int di) {
         const int V = L * d.O;
-        host[di].assign((size_t)std::max(V, 1), 0.0);
-        if (V == 0) continue;
+        host[di].assign((size_t)V, 0.0);
         cudaStream_t st = d.stream;
-        CU_TRY(cudaEventRecord(d.ev[0], st));
+        RC_TRY(mark(d, MARK_BEGIN, st));
         RC_TRY(d.lam_dev.ensure((size_t)L * ng * sizeof(double)));
         CU_TRY(cudaMemcpyAsync(d.lam_dev.p, lams, (size_t)L * ng * sizeof(double), cudaMemcpyHostToDevice, st));
         BatchMap<Real> bm;
@@ -1398,44 +1414,37 @@ static int sweep_impl(bpltv_ctx *ctx, const double *lams, int L, int lm, int ln,
             amap = d.amap.as<Real>();
         }
         d.launches += 1;
-        CU_TRY(cudaEventRecord(d.ev[1], st));
-        const Real *u = nullptr; int used = 0, depth = 1;
-        RC_TRY(run_pdps<Real>(d, d.noisy.as<Real>(), M, N, V, 0.0, amap, o, st, &u, &used, &depth, &bm));
+        RC_TRY(mark(d, MARK_UPLOAD, st));
+        int used = 0, depth = 1;
+        RC_TRY(run_pdps<Real>(d, d.noisy.as<Real>(), M, N, V, 0.0, amap, o, st, &us[di], &used, &depth, &bm));
         ctx->stats.pdps_kernel_used = used;
         ctx->stats.tblock_depth = depth;
-        CU_TRY(cudaEventRecord(d.ev[2], st));
+        RC_TRY(mark(d, MARK_SOLVE, st));
         RC_TRY(d.partials.ensure(std::max<size_t>((size_t)V, 1024) * sizeof(double)));
-        sqerr_image_kernel<Real><<<V, 256, 0, st>>>(u, d.truth.as<Real>(), (int)plane, d.O, d.partials.as<double>());
+        sqerr_image_kernel<Real><<<V, 256, 0, st>>>(us[di], d.truth.as<Real>(), (int)plane, d.O, d.partials.as<double>());
         d.launches += 1;
         CU_TRY(cudaMemcpyAsync(host[di].data(), d.partials.p, (size_t)V * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CU_TRY(cudaEventRecord(d.ev[3], st));
+        return mark(d, MARK_COST, st);
+    };
+    auto download = [&](Dev &d, int di) {
         if (u_out)
             for (int l = 0; l < L; ++l)
-                RC_TRY(download_stack<Real>(d, u + (size_t)l * d.O * plane, plane * d.O,
-                                            u_out + ((size_t)l * O + d.o_begin) * plane, st));
-        CU_TRY(cudaEventRecord(d.ev[4], st));
-    }
-    for (int l = 0; l < L; ++l) cost_out[l] = 0.0;
-    for (int di = 0; di < ndev; ++di) {  // fixed device and image order: deterministic sums
-        Dev &d = ctx->devs[di];
-        if (L * d.O == 0) continue;
-        CU_TRY(cudaSetDevice(d.id));
-        CU_TRY(cudaStreamSynchronize(d.stream));
+                RC_TRY(download_stack<Real>(d, us[di] + (size_t)l * d.O * plane, plane * d.O,
+                                            u_out + ((size_t)l * O + d.o_begin) * plane, d.stream));
+        return mark(d, MARK_DOWNLOAD, d.stream);
+    };
+    auto fold = [&](Dev &d, int di) {      // image order within the device: deterministic sums
         for (int l = 0; l < L; ++l)
             for (int oo = 0; oo < d.O; ++oo) {
                 const double v = host[di][(size_t)l * d.O + oo];
-                cost_out[l] += v;
+                cost[l] += v;
                 if (sqerr_out) sqerr_out[(size_t)l * O + d.o_begin + oo] = v;
             }
-        ctx->stats.ms_upload = std::max<double>(ctx->stats.ms_upload, ev_ms(d.ev[0], d.ev[1]));
-        ctx->stats.ms_pdps = std::max<double>(ctx->stats.ms_pdps, ev_ms(d.ev[1], d.ev[2]));
-        ctx->stats.ms_cost = std::max<double>(ctx->stats.ms_cost, ev_ms(d.ev[2], d.ev[3]));
-        ctx->stats.ms_download = std::max<double>(ctx->stats.ms_download, ev_ms(d.ev[3], d.ev[4]));
-        ctx->stats.ms_total = std::max<double>(ctx->stats.ms_total, ev_ms(d.ev[0], d.ev[4]));
-        ctx->stats.kernel_launches += d.launches;
-    }
+        fold_device_stats(ctx->stats, d);
+    };
+    RC_TRY(run_sharded(ctx, true, enqueue, download, fold));
     for (int l = 0; l < L; ++l) {
-        cost_out[l] *= 0.5;
+        cost_out[l] = 0.5 * cost[l];
         if (!std::isfinite(cost_out[l])) return fail(BPLTV_ERR_NUMERIC, "non-finite cost for parameter set %d", l);
     }
     ctx->stats.pdps_iterations = o.maxiter;
@@ -1454,44 +1463,31 @@ static int gradient_impl(bpltv_ctx *ctx, const double *u_host, const double *lam
     std::memset(&ctx->stats, 0, sizeof ctx->stats);
     std::vector<std::vector<double>> host(ndev, std::vector<double>(ng, 0.0));
     std::vector<double> relres(ndev, 0.0);
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        CU_TRY(cudaSetDevice(d.id));
-        d.launches = 0;
-        d.grad_used_nd = d.grad_used_band = false;
-        if (d.O == 0) continue;
+    std::vector<double> grad(ng, 0.0);
+    auto enqueue = [&](Dev &d, int di) {
         cudaStream_t st = d.stream;
         RC_TRY(d.scalars.ensure((1 + ng) * sizeof(double)));
         RC_TRY(upload_stack<Real>(d, u_host + plane * d.o_begin, plane * d.O, d.ubuf, st));
         double alpha_s; const Real *amap;
         RC_TRY(prepare_lambda<Real>(d, lam, lm, ln, d.M, d.N, st, &alpha_s, &amap));
-        CU_TRY(cudaEventRecord(d.ev[2], st));
-        GradProblem<Real> gp;
-        gp.u = d.ubuf.as<Real>(); gp.ubar = d.truth.as<Real>(); gp.M = d.M; gp.N = d.N; gp.O = d.O;
-        gp.alpha_s = alpha_s; gp.alpha_map = amap; gp.lm = lm; gp.ln = ln; gp.regularised = regularised != 0;
-        gp.gamma = eo.gamma; gp.act_tol = eo.act_tol;
-        gp.eps_act = eo.eps_act > 0 ? eo.eps_act : (ng == 1 ? 2.220446049250313e-16 : 1.4901161193847656e-08);
-        gp.tol = eo.solver_tol; gp.maxit = eo.solver_maxit; gp.solver = eo.solver;
+        RC_TRY(mark(d, MARK_BEGIN, st));
+        const GradProblem<Real> gp = tv_grad_problem<Real>(d, d.ubuf.as<Real>(), alpha_s, amap, lm, ln, regularised != 0, eo);
         CU_TRY(cudaMemsetAsync(d.scalars.p, 0, (1 + ng) * sizeof(double), st));
-        int rc = run_tv_gradient<Real>(d, gp, st, d.scalars.as<double>() + 1);
+        const int rc = run_tv_gradient<Real>(d, gp, st, d.scalars.as<double>() + 1);
         if (rc != 0) return fail(rc, "gradient: %s", d.grad.err.c_str());
-        CU_TRY(cudaEventRecord(d.ev[3], st));
+        RC_TRY(mark(d, MARK_GRADIENT, st));
         CU_TRY(cudaMemcpyAsync(host[di].data(), d.scalars.as<double>() + 1, ng * sizeof(double), cudaMemcpyDeviceToHost, st));
         if (relres_of_last_gradient(d))
             CU_TRY(cudaMemcpyAsync(&relres[di], relres_of_last_gradient(d), sizeof(double), cudaMemcpyDeviceToHost, st));
-    }
-    std::vector<double> grad(ng, 0.0);
-    for (int di = 0; di < ndev; ++di) {
-        Dev &d = ctx->devs[di];
-        if (d.O == 0) continue;
-        CU_TRY(cudaSetDevice(d.id));
-        CU_TRY(cudaStreamSynchronize(d.stream));
+        return 0;
+    };
+    auto fold = [&](Dev &d, int di) {
         for (int k = 0; k < ng; ++k) grad[k] += host[di][k];
-        ctx->stats.ms_gradient = std::max<double>(ctx->stats.ms_gradient, ev_ms(d.ev[2], d.ev[3]));
-        ctx->stats.kernel_launches += d.launches;
+        fold_device_stats(ctx->stats, d);
         ctx->stats.solver_iterations += d.grad.last_iterations;
         ctx->stats.solver_max_relres = std::max(ctx->stats.solver_max_relres, relres[di]);
-    }
+    };
+    RC_TRY(run_sharded(ctx, true, enqueue, no_download, fold));
     ctx->stats.n_devices = ndev;
     for (int k = 0; k < ng; ++k) {
         if (!std::isfinite(grad[k]))
@@ -1709,6 +1705,25 @@ static int check_shape(int M, int N, int O)
     return 0;
 }
 
+// denoise(noisy = NULL) takes the resident dataset: there must be one, of the call's shape
+static int check_resident_shape(const bpltv_ctx *ctx, const double *noisy, int M, int N, int O)
+{
+    if (noisy) return 0;
+    if (!ctx->have_dataset) return fail(BPLTV_ERR_STATE, "denoise(noisy=NULL) needs bpltv_set_dataset first");
+    if (M != ctx->M || N != ctx->N || O != ctx->O)
+        return fail(BPLTV_ERR_ARG, "shape %dx%dx%d does not match the resident dataset %dx%dx%d", M, N, O, ctx->M,
+                    ctx->N, ctx->O);
+    return 0;
+}
+
+// the sum-of-regularisers parameter: three lm×ln grids, one after the other
+static int check_lambda3(const double *lam, int lm, int ln)
+{
+    if (!lam || lm < 1 || ln < 1) return fail(BPLTV_ERR_ARG, "lambda grid must be at least 1x1(x3)");
+    for (int k = 0; k < 3; ++k) RC_TRY(check_lambda(lam + (size_t)k * lm * ln, lm, ln));
+    return 0;
+}
+
 int bpltv_set_dataset(bpltv_ctx *ctx, const double *truth, const double *noisy, int M, int N, int O)
 {
     if (!ctx || !truth || !noisy) return fail(BPLTV_ERR_ARG, "NULL argument");
@@ -1726,34 +1741,32 @@ int bpltv_denoise(bpltv_ctx *ctx, const double *noisy, int M, int N, int O, cons
     bpltv_pdps_opts o;
     if (opts) o = *opts; else bpltv_default_pdps_opts(&o);
     RC_TRY(check_pdps_opts(o));
-    if (!noisy) {
-        if (!ctx->have_dataset) return fail(BPLTV_ERR_STATE, "denoise(noisy=NULL) needs bpltv_set_dataset first");
-        if (M != ctx->M || N != ctx->N || O != ctx->O)
-            return fail(BPLTV_ERR_ARG, "shape %dx%dx%d does not match the resident dataset %dx%dx%d", M, N, O, ctx->M,
-                        ctx->N, ctx->O);
-    }
+    RC_TRY(check_resident_shape(ctx, noisy, M, N, O));
     return ctx->prec == 64 ? denoise_impl<double>(ctx, noisy, M, N, O, lam, lm, ln, o, u_out)
                            : denoise_impl<float>(ctx, noisy, M, N, O, lam, lm, ln, o, u_out);
 }
 
-static int check_eval(bpltv_ctx *ctx, const double *lam, int lm, int ln, const bpltv_eval_opts *opts,
+// Arguments of an evaluation on the resident dataset: the TV learning function (sets = 1) or the sum of regularisers
+// (sets = 3 λ grids).  force_branch == 3 evaluates the loss alone (λ-sweeps, validation): no gradient is formed, so
+// λ > 0 does not apply, nor, on the TV path, the reference's square-image precondition.
+static int check_eval(bpltv_ctx *ctx, const double *lam, int lm, int ln, int sets, const bpltv_eval_opts *opts,
                       bpltv_eval_opts &eo)
 {
     if (!ctx) return fail(BPLTV_ERR_ARG, "NULL context");
     if (!ctx->have_dataset) return fail(BPLTV_ERR_STATE, "no resident dataset: call bpltv_set_dataset first");
-    RC_TRY(check_lambda(lam, lm, ln));
-    if (opts) eo = *opts; else bpltv_default_eval_opts(&eo);
+    RC_TRY(sets == 1 ? check_lambda(lam, lm, ln) : check_lambda3(lam, lm, ln));
+    if (opts) eo = *opts;
+    else if (sets == 1) bpltv_default_eval_opts(&eo);
+    else bpltv_default_sumregs_eval_opts(&eo);
     RC_TRY(check_pdps_opts(eo.pdps));
-    // force_branch == 3 evaluates the loss alone (λ-sweeps, validation): no gradient is formed, so neither the
-    // reference's square-image precondition nor λ > 0 applies (like the sum-of-regularisers path)
     const bool grad_needed = eo.force_branch != 3;
-    if (grad_needed && ctx->M != ctx->N)
-        return fail(BPLTV_ERR_ARG, "the gradient assumes square images like the reference "
-                                   "(TVLearningFunctionVec.jl:102); got %dx%d", ctx->M, ctx->N);
+    if ((grad_needed || sets == 3) && ctx->M != ctx->N)
+        return fail(BPLTV_ERR_ARG, "the gradient assumes square images like the reference (%s); got %dx%d",
+                    sets == 1 ? "TVLearningFunctionVec.jl:102" : "SumRegsLearningFunction.jl:116", ctx->M, ctx->N);
     if (lm > ctx->M || ln > ctx->N) return fail(BPLTV_ERR_ARG, "lambda grid larger than the image");
-    for (int k = 0; k < lm * ln; ++k)
-        if (grad_needed ? !(lam[k] > 0.0) : !(lam[k] >= 0.0))
-            return fail(BPLTV_ERR_ARG, grad_needed ? "lambda[%d] must be > 0 for the gradient" : "lambda[%d] must be >= 0", k);
+    if (grad_needed)
+        for (int k = 0; k < sets * lm * ln; ++k)
+            if (!(lam[k] > 0.0)) return fail(BPLTV_ERR_ARG, "lambda[%d] must be > 0 for the gradient", k);
     if (!(eo.gamma > 0) || !(eo.act_tol >= 0)) return fail(BPLTV_ERR_ARG, "bad gamma / act_tol");
     return 0;
 }
@@ -1762,7 +1775,7 @@ int bpltv_learn_eval(bpltv_ctx *ctx, const double *lam, int lm, int ln, double D
                      double *u_out, double *cost_out, double *grad_out)
 {
     bpltv_eval_opts eo;
-    RC_TRY(check_eval(ctx, lam, lm, ln, opts, eo));
+    RC_TRY(check_eval(ctx, lam, lm, ln, 1, opts, eo));
     if (!cost_out || !grad_out) return fail(BPLTV_ERR_ARG, "NULL output");
     return ctx->prec == 64 ? learn_eval_impl<double>(ctx, lam, lm, ln, Delta, eo, u_out, cost_out, grad_out)
                            : learn_eval_impl<float>(ctx, lam, lm, ln, Delta, eo, u_out, cost_out, grad_out);
@@ -1772,7 +1785,7 @@ int bpltv_gradient(bpltv_ctx *ctx, const double *u, const double *lam, int lm, i
                    const bpltv_eval_opts *opts, double *grad_out)
 {
     bpltv_eval_opts eo;
-    RC_TRY(check_eval(ctx, lam, lm, ln, opts, eo));
+    RC_TRY(check_eval(ctx, lam, lm, ln, 1, opts, eo));
     if (!u || !grad_out) return fail(BPLTV_ERR_ARG, "NULL argument");
     return ctx->prec == 64 ? gradient_impl<double>(ctx, u, lam, lm, ln, regularised, eo, grad_out)
                            : gradient_impl<float>(ctx, u, lam, lm, ln, regularised, eo, grad_out);
@@ -1809,47 +1822,21 @@ int bpltv_sumregs_denoise(bpltv_ctx *ctx, const double *noisy, int M, int N, int
 {
     if (!ctx || !u_out) return fail(BPLTV_ERR_ARG, "NULL argument");
     RC_TRY(check_shape(M, N, O));
-    if (!lam || lm < 1 || ln < 1) return fail(BPLTV_ERR_ARG, "lambda grid must be at least 1x1(x3)");
-    for (int k = 0; k < 3; ++k) RC_TRY(check_lambda(lam + (size_t)k * lm * ln, lm, ln));
+    RC_TRY(check_lambda3(lam, lm, ln));
     bpltv_pdps_opts o;
     if (opts) o = *opts;
     else { bpltv_eval_opts e; bpltv_default_sumregs_eval_opts(&e); o = e.pdps; }
     RC_TRY(check_pdps_opts(o));
-    if (!noisy) {
-        if (!ctx->have_dataset) return fail(BPLTV_ERR_STATE, "denoise(noisy=NULL) needs bpltv_set_dataset first");
-        if (M != ctx->M || N != ctx->N || O != ctx->O)
-            return fail(BPLTV_ERR_ARG, "shape %dx%dx%d does not match the resident dataset %dx%dx%d", M, N, O, ctx->M,
-                        ctx->N, ctx->O);
-    }
+    RC_TRY(check_resident_shape(ctx, noisy, M, N, O));
     return ctx->prec == 64 ? sumregs_denoise_impl<double>(ctx, noisy, M, N, O, lam, lm, ln, o, u_out)
                            : sumregs_denoise_impl<float>(ctx, noisy, M, N, O, lam, lm, ln, o, u_out);
-}
-
-static int check_sumregs_eval(bpltv_ctx *ctx, const double *lam, int lm, int ln, const bpltv_eval_opts *opts,
-                              bpltv_eval_opts &eo)
-{
-    if (!ctx) return fail(BPLTV_ERR_ARG, "NULL context");
-    if (!ctx->have_dataset) return fail(BPLTV_ERR_STATE, "no resident dataset: call bpltv_set_dataset first");
-    if (!lam || lm < 1 || ln < 1) return fail(BPLTV_ERR_ARG, "lambda grid must be at least 1x1(x3)");
-    for (int k = 0; k < 3; ++k) RC_TRY(check_lambda(lam + (size_t)k * lm * ln, lm, ln));
-    if (opts) eo = *opts; else bpltv_default_sumregs_eval_opts(&eo);
-    RC_TRY(check_pdps_opts(eo.pdps));
-    if (ctx->M != ctx->N)
-        return fail(BPLTV_ERR_ARG, "the gradient assumes square images like the reference "
-                                   "(SumRegsLearningFunction.jl:116); got %dx%d", ctx->M, ctx->N);
-    if (lm > ctx->M || ln > ctx->N) return fail(BPLTV_ERR_ARG, "lambda grid larger than the image");
-    if (eo.force_branch != 3)
-        for (int k = 0; k < 3 * lm * ln; ++k)
-            if (!(lam[k] > 0.0)) return fail(BPLTV_ERR_ARG, "lambda[%d] must be > 0 for the gradient", k);
-    if (!(eo.gamma > 0) || !(eo.act_tol >= 0)) return fail(BPLTV_ERR_ARG, "bad gamma / act_tol");
-    return 0;
 }
 
 int bpltv_sumregs_learn_eval(bpltv_ctx *ctx, const double *lam, int lm, int ln, double Delta,
                              const bpltv_eval_opts *opts, double *u_out, double *cost_out, double *grad_out)
 {
     bpltv_eval_opts eo;
-    RC_TRY(check_sumregs_eval(ctx, lam, lm, ln, opts, eo));
+    RC_TRY(check_eval(ctx, lam, lm, ln, 3, opts, eo));
     if (!cost_out || !grad_out) return fail(BPLTV_ERR_ARG, "NULL output");
     return ctx->prec == 64
                ? sumregs_learn_eval_impl<double>(ctx, lam, lm, ln, Delta, eo, nullptr, u_out, cost_out, grad_out)
@@ -1860,7 +1847,7 @@ int bpltv_sumregs_gradient(bpltv_ctx *ctx, const double *u, const double *lam, i
                            const bpltv_eval_opts *opts, double *grad_out)
 {
     bpltv_eval_opts eo;
-    RC_TRY(check_sumregs_eval(ctx, lam, lm, ln, opts, eo));
+    RC_TRY(check_eval(ctx, lam, lm, ln, 3, opts, eo));
     if (!u || !grad_out) return fail(BPLTV_ERR_ARG, "NULL argument");
     eo.force_branch = regularised ? 2 : 1;
     return ctx->prec == 64
@@ -1876,14 +1863,19 @@ static int single_dev(bpltv_ctx *ctx)
     return 0;
 }
 
+static int check_aligned16(const void *a, const void *b)
+{
+    if (((uintptr_t)a | (uintptr_t)b) & 15)
+        return fail(BPLTV_ERR_ARG, "device pointers must be 16-byte aligned (vector and TMA accesses)");
+    return 0;
+}
 
 int bpltv_denoise_device(bpltv_ctx *ctx, const void *d_noisy, int M, int N, int O, const double *lam, int lm, int ln,
                          const bpltv_pdps_opts *opts, void *d_u_out, void *stream)
 {
     RC_TRY(single_dev(ctx));
     if (!d_noisy || !d_u_out) return fail(BPLTV_ERR_ARG, "NULL device pointer");
-    if (((uintptr_t)d_noisy | (uintptr_t)d_u_out) & 15)
-        return fail(BPLTV_ERR_ARG, "device pointers must be 16-byte aligned (vector and TMA accesses)");
+    RC_TRY(check_aligned16(d_noisy, d_u_out));
     RC_TRY(check_shape(M, N, O));
     RC_TRY(check_lambda(lam, lm, ln));
     bpltv_pdps_opts o;
@@ -1899,8 +1891,7 @@ int bpltv_set_dataset_device(bpltv_ctx *ctx, const void *d_truth, const void *d_
 {
     RC_TRY(single_dev(ctx));
     if (!d_truth || !d_noisy) return fail(BPLTV_ERR_ARG, "NULL device pointer");
-    if (((uintptr_t)d_truth | (uintptr_t)d_noisy) & 15)
-        return fail(BPLTV_ERR_ARG, "device pointers must be 16-byte aligned (vector and TMA accesses)");
+    RC_TRY(check_aligned16(d_truth, d_noisy));
     RC_TRY(check_shape(M, N, O));
     Dev &d = ctx->devs[0];
     CU_TRY(cudaSetDevice(d.id));
@@ -1923,7 +1914,7 @@ int bpltv_learn_eval_device(bpltv_ctx *ctx, const double *lam, int lm, int ln, d
 {
     RC_TRY(single_dev(ctx));
     bpltv_eval_opts eo;
-    RC_TRY(check_eval(ctx, lam, lm, ln, opts, eo));
+    RC_TRY(check_eval(ctx, lam, lm, ln, 1, opts, eo));
     if (!d_costgrad) return fail(BPLTV_ERR_ARG, "NULL d_costgrad");
     cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->devs[0].stream;
     return ctx->prec == 64 ? learn_eval_device_impl<double>(ctx, lam, lm, ln, Delta, eo, d_u_out, d_costgrad, st)

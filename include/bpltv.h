@@ -132,7 +132,9 @@ void bpltv_default_eval_opts(bpltv_eval_opts *o);
  * dataset on each listed device.  precision: 64 (reference arithmetic) or 32.
  * device_ids == NULL → device 0..ndev-1.  Images are sharded over the devices in
  * contiguous blocks along O (SURVEY §8e); partial costs/gradients are summed on
- * the host in device order (single process: no collective is needed).           */
+ * the host in device order (single process: no collective is needed).  A device
+ * id may repeat, and each entry is its own shard: tests/test_gpu_sharded.py runs
+ * the sharded path on one GPU with [0, 0].                                       */
 int bpltv_create(const int *device_ids, int ndev, int precision, bpltv_ctx **out);
 int bpltv_destroy(bpltv_ctx *ctx);
 
