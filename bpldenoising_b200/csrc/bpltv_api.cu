@@ -1118,23 +1118,32 @@ static int set_dataset_impl(bpltv_ctx *ctx, const double *truth, const double *n
 // (gradient_nd.cuh: O(n³) operations, the whole GPU per image); 1 — the banded factorisations of round 1 (multiplier-
 // space Cholesky for `gradient`, node-space LU for `gradient_reg`), kept as an independent second implementation.
 // BPLTV_GRAD_SOLVER overrides option 0.
+// A shape that neither the shared-memory front kernels nor the band solvers take goes back to the nested-dissection
+// solver with its large-front variants (fronts beyond shared memory).
 template <typename Real>
 static int run_tv_gradient(Dev &d, const GradProblem<Real> &gp, cudaStream_t st, double *d_grad_out)
 {
     int solver = gp.solver;
     if (solver == 0) solver = env_int("BPLTV_GRAD_SOLVER", 0);
     d.last_grad = Dev::GRAD_NONE;
-    if (solver != 1) {
+    auto nd = [&](bool large) {
         if (!d.nd) d.nd = nd_work_create();
         NdProblem np;
         np.u = gp.u; np.ubar = gp.ubar; np.prec = (int)sizeof(Real) * 8; np.M = gp.M; np.N = gp.N; np.O = gp.O;
         np.alpha_s = gp.alpha_s; np.alpha_map = gp.alpha_map; np.lm = gp.lm; np.ln = gp.ln; np.regularised = gp.regularised;
         np.gamma = gp.gamma; np.act_tol = gp.act_tol; np.eps_act = gp.eps_act; np.tol = gp.tol; np.maxit = gp.maxit;
+        np.large_fronts = large;
         const int rc = nd_run_gradient(d.nd, np, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
-        if (rc == 0) { d.last_grad = Dev::GRAD_TV_ND; return 0; }
-        if (rc != -1) { d.grad.err = nd_work_error(d.nd); return rc; }
+        if (rc == 0) d.last_grad = Dev::GRAD_TV_ND;
+        else if (rc != -1) d.grad.err = nd_work_error(d.nd);
+        return rc;
+    };
+    if (solver != 1) {
+        const int rc = nd(false);
+        if (rc != -1) return rc;
         // -1: fronts beyond shared memory for this image size — the band solver takes over
     }
+    int rc = -1;
     const char *lu_env = bpltv::env_get("BPLTV_GRAD_REG_LU");
     const bool lu = lu_env && *lu_env ? atoi(lu_env) != 0 : true;
     if (gp.regularised && lu && gp.M == gp.N && gp.M >= 4) {
@@ -1142,12 +1151,15 @@ static int run_tv_gradient(Dev &d, const GradProblem<Real> &gp, cudaStream_t st,
         lp.u = gp.u; lp.ubar = gp.ubar; lp.M = gp.M; lp.N = gp.N; lp.O = gp.O;
         lp.alpha[0] = gp.alpha_s; lp.alpha[1] = lp.alpha[2] = 0.0;
         lp.alpha_maps = gp.alpha_map; lp.lm = gp.lm; lp.ln = gp.ln; lp.gamma = gp.gamma; lp.nops = 1;
-        const int rc = run_gradient_lu<Real>(d.grad, lp, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
+        rc = run_gradient_lu<Real>(d.grad, lp, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
         if (rc == 0) d.last_grad = Dev::GRAD_TV_BAND;
-        if (rc != -1) return rc;      // -1: the LU does not take this shape (panels beyond shared memory): Cholesky
+        // -1: the LU does not take this shape (panels beyond shared memory): Cholesky
     }
-    const int rc = run_gradient<Real>(d.grad, gp, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
-    if (rc == 0) d.last_grad = Dev::GRAD_TV_BAND;
+    if (rc == -1) {
+        rc = run_gradient<Real>(d.grad, gp, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
+        if (rc == 0) d.last_grad = Dev::GRAD_TV_BAND;
+    }
+    if (rc == -1 && solver != 1 && gp.M == gp.N) return nd(true);
     return rc;
 }
 
@@ -1156,35 +1168,49 @@ static int run_tv_gradient(Dev &d, const GradProblem<Real> &gp, cudaStream_t st,
 // patch :330-407) is the same in multiplier space (3-6 unknowns per pixel): both take the nested-dissection
 // multifrontal Cholesky.  Solver 1, the patch sumregs_gradient_reg, a shape the fronts do not take (-1) or one that
 // does not fit in memory go to the node-space band LU / compliance-form band Cholesky of run_gradient3, which needs
-// less memory per image.
+// less memory per image.  A shape the band solvers refuse as well (above 430² for the band LU, 136² for the band
+// Cholesky) goes back to the fronts with their large-front variants; a failure there is final, and an image whose
+// workspace does not fit returns BPLTV_ERR_ALLOC with the size it needs.
 template <typename Real>
 static int run_sumregs_gradient(Dev &d, const Grad3Problem<Real> &gp, int solver, int maxit, cudaStream_t st,
                                 double *d_grad_out)
 {
     if (solver == 0) solver = env_int("BPLTV_GRAD_SOLVER", 0);
     d.last_grad = Dev::GRAD_NONE;
-    if (solver != 1 && gp.M == gp.N && !(gp.regularised && gp.alpha_maps)) {
+    const bool fronts = solver != 1 && gp.M == gp.N && !(gp.regularised && gp.alpha_maps);
+    auto nd = [&](bool large) {
         if (!d.nd3) d.nd3 = nd_work_create();
         int rc;
         if (gp.regularised) {
             Nd3Problem np;
             np.u = gp.u; np.ubar = gp.ubar; np.prec = (int)sizeof(Real) * 8; np.M = gp.M; np.N = gp.N; np.O = gp.O;
             for (int k = 0; k < 3; ++k) np.alpha[k] = gp.alpha[k];
-            np.gamma = gp.gamma; np.tol = 0.0; np.maxit = maxit;
+            np.gamma = gp.gamma; np.tol = 0.0; np.maxit = maxit; np.large_fronts = large;
             rc = nd_run_gradient3_reg(d.nd3, np, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
         } else {
             Nd3mProblem np;
             np.u = gp.u; np.ubar = gp.ubar; np.alpha_maps = gp.alpha_maps; np.prec = (int)sizeof(Real) * 8;
             np.M = gp.M; np.N = gp.N; np.O = gp.O; np.lm = gp.lm; np.ln = gp.ln;
             for (int k = 0; k < 3; ++k) np.alpha[k] = gp.alpha[k];
-            np.act_tol = gp.act_tol; np.eps_act = gp.eps_act; np.tol = 0.0; np.maxit = maxit;
+            np.act_tol = gp.act_tol; np.eps_act = gp.eps_act; np.tol = 0.0; np.maxit = maxit; np.large_fronts = large;
             rc = nd_run_gradient3(d.nd3, np, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
         }
-        if (rc == 0) { d.last_grad = Dev::GRAD_SR_ND; return 0; }
-        if (rc != -1 && rc != BPLTV_ERR_ALLOC) { d.grad3.err = nd_work_error(d.nd3); return rc; }
+        if (rc == 0) d.last_grad = Dev::GRAD_SR_ND;
+        return rc;
+    };
+    int nd_rc = -1;
+    if (fronts) {
+        nd_rc = nd(false);
+        if (nd_rc == 0) return 0;
+        if (nd_rc != -1 && nd_rc != BPLTV_ERR_ALLOC) { d.grad3.err = nd_work_error(d.nd3); return nd_rc; }
     }
-    const int rc = run_gradient3<Real>(d.grad3, gp, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
+    int rc = run_gradient3<Real>(d.grad3, gp, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
     if (rc == 0) d.last_grad = Dev::GRAD_SR_BAND;
+    if (rc == -1 && fronts) {
+        if (nd_rc == -1) rc = nd(true);
+        else rc = nd_rc;        // the fronts took the shape but their workspace did not fit: say so, with its size
+        if (rc != 0 && rc != -1) d.grad3.err = nd_work_error(d.nd3);
+    }
     return rc;
 }
 

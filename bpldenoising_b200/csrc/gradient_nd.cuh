@@ -7,8 +7,10 @@
 // spreads over the SMs level by level and many images fill the GPU together.
 #pragma once
 #include <cstring>
+#include <map>
 #include <mutex>
 #include <string>
+#include <tuple>
 #include <unordered_map>
 #include <vector>
 
@@ -74,7 +76,7 @@ struct NdBuf {
 struct NdWork {
     std::string err;
     NdPlan plan;
-    NdBuf pix, off, off3, lvl, vec, posg, foff, totals, ast, L, U0, U1, UV0, UV1, info, out_img, relres, relres_max;
+    NdBuf pix, off, off3, lvl, vec, posg, foff, totals, ast, L, U0, U1, UV0, UV1, scr, info, out_img, relres, relres_max;
     std::vector<long long> h_totals;
     size_t budget_cached = 0;
     // what the last call saw (statistics)
@@ -87,7 +89,7 @@ struct NdWork {
     {
         slots_key_n = slots_key_node = slots_key_want = -1;
         plan.release();
-        NdBuf *all[] = {&pix, &off, &off3, &lvl, &vec, &posg, &foff, &totals, &ast, &L, &U0, &U1, &UV0, &UV1, &info, &out_img, &relres, &relres_max};
+        NdBuf *all[] = {&pix, &off, &off3, &lvl, &vec, &posg, &foff, &totals, &ast, &L, &U0, &U1, &UV0, &UV1, &scr, &info, &out_img, &relres, &relres_max};
         for (NdBuf *b : all) b->release();
     }
 };
@@ -139,15 +141,17 @@ static inline int nd_fail(NdWork &w, int code, const std::string &msg) { w.err =
 
 // Opt-in shared memory of the front kernels.  -1: a front does not fit (the caller falls back to a band solver).
 static int nd_kernel_attributes(NdWork &w, size_t fsmem, size_t ssmem, size_t fsmem_small, size_t ssmem_small, size_t smem_optin,
-                                size_t fsmem8 = 0)      // fsmem8: of the levels that take 8-column block steps
+                                size_t fsmem8 = 0,      // fsmem8: of the levels that take 8-column block steps
+                                size_t fsmem_large = 0, size_t ssmem_large = 0)     // of the levels on the large-front variants
 {
-    if (fsmem > smem_optin || ssmem > smem_optin || fsmem_small > smem_optin || ssmem_small > smem_optin || fsmem8 > smem_optin)
+    if (fsmem > smem_optin || ssmem > smem_optin || fsmem_small > smem_optin || ssmem_small > smem_optin || fsmem8 > smem_optin ||
+        fsmem_large > smem_optin || ssmem_large > smem_optin)
         return -1;      // the caller falls back to the band solver
     {
         // the opt-in shared-memory size is an attribute of the KERNEL on the current device, shared by every workspace
         // that launches it (the TV solver and the sum-of-regularisers one): raised to the largest any of them asked for
         static std::mutex mu;
-        static int have[64][6] = {};
+        static int have[64][8] = {};
         int dev = 0;
         cudaGetDevice(&dev);
         dev = std::max(0, std::min(63, dev));
@@ -168,6 +172,18 @@ static int nd_kernel_attributes(NdWork &w, size_t fsmem, size_t ssmem, size_t fs
             if (e == cudaSuccess) e = cudaFuncSetAttribute(nd_factor8_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
             if (e == cudaSuccess) have[dev][5] = (int)fsmem8;
         }
+        if (e == cudaSuccess && fsmem_large > 0 && have[dev][6] < (int)fsmem_large) {
+            for (auto k : {nd_factor_large_kernel, nd_factor8_large_kernel, nd_factor_large_cluster_kernel, nd_factor8_large_cluster_kernel})
+                if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsmem_large);
+            for (auto k : {nd_factor_large_cluster_kernel, nd_factor8_large_cluster_kernel})
+                if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+            if (e == cudaSuccess) have[dev][6] = (int)fsmem_large;
+        }
+        if (e == cudaSuccess && ssmem_large > 0 && have[dev][7] < (int)ssmem_large) {
+            e = cudaFuncSetAttribute(nd_fwd_large_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssmem_large);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(nd_bwd_large_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssmem_large);
+            if (e == cudaSuccess) have[dev][7] = (int)ssmem_large;
+        }
         if (e == cudaSuccess && have[dev][1] < (int)ssmem) {
             e = cudaFuncSetAttribute(nd_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssmem);
             if (e == cudaSuccess) e = cudaFuncSetAttribute(nd_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssmem);
@@ -184,16 +200,45 @@ static int nd_kernel_attributes(NdWork &w, size_t fsmem, size_t ssmem, size_t fs
         }
         if (e != cudaSuccess) {
             cudaGetLastError();
-            return nd_fail(w, -2, std::string("nested-dissection kernel attributes: ") + cudaGetErrorString(e));
+            char buf[160];
+            snprintf(buf, sizeof buf, " (dynamic shared memory: factor %zu / %zu / %zu B, solves %zu / %zu B)", fsmem, fsmem8,
+                     fsmem_large, ssmem, ssmem_large);
+            return nd_fail(w, -2, std::string("nested-dissection kernel attributes: ") + cudaGetErrorString(e) + buf);
         }
     }
     return 0;
 }
 
+// Dynamic shared memory a front kernel may ask for: the opt-in maximum per block less the static shared memory of the
+// factorisation kernels (their block-step flags, 16 B), which the opt-in maximum also has to hold.
+static size_t nd_dynamic_optin(size_t smem_optin)
+{
+    static const size_t stat = [] {
+        size_t m = 0;
+        for (auto k : {nd_factor_kernel, nd_factor8_kernel, nd_factor_cluster_kernel, nd_factor8_cluster_kernel, nd_factor_large_kernel,
+                       nd_factor8_large_kernel, nd_factor_large_cluster_kernel, nd_factor8_large_cluster_kernel}) {
+            cudaFuncAttributes a;
+            if (cudaFuncGetAttributes(&a, k) == cudaSuccess) m = std::max(m, a.sharedSizeBytes);
+            else cudaGetLastError();
+        }
+        return m;
+    }();
+    return smem_optin > stat ? smem_optin - stat : 0;
+}
+
+// Shared memory (bytes) beyond which a level takes the large-front variants: the opt-in maximum.  Test hook:
+// BPLTV_ND_LARGE_KB lowers it, so that small images run the variants where the shared-memory kernels can be compared.
+static size_t nd_large_limit(size_t smem_optin)
+{
+    const char *e = bpltv::env_get("BPLTV_ND_LARGE_KB");
+    return e && *e ? std::min<size_t>(smem_optin, (size_t)std::max(0, atoi(e)) << 10) : smem_optin;
+}
+
 // Launch plan of every level of the tree for `mb` unknowns per pixel at most (`fsz` typical): CTA sizes, shared memory of
 // the largest front (worst case: mb unknowns on every pixel), kernel attributes.  -1: a front does not fit in shared
-// memory (the caller falls back to a band solver).
-static int nd_prepare_levels(NdWork &w, const NdSymbolic &sym, int mb, double fsz, int O, size_t smem_optin,
+// memory and `large` is not set (the caller lets a band solver try first); with `large`, such levels take the
+// large-front variants.
+static int nd_prepare_levels(NdWork &w, const NdSymbolic &sym, int mb, double fsz, int O, size_t smem_optin, bool large,
                              std::vector<NdLevelPlan> &plan, std::vector<char> &plan_small)
 {
     const int nsteps = sym.nsteps();
@@ -208,16 +253,29 @@ static int nd_prepare_levels(NdWork &w, const NdSymbolic &sym, int mb, double fs
     const int cta_threads_s = e2 && *e2 ? std::max(64, std::min(512, atoi(e2))) : 512;
     plan.assign(nsteps, NdLevelPlan());
     plan_small.assign(nsteps, 0);
-    size_t fsmem = 0, ssmem = 0, fsmem_small = 0, ssmem_small = 0;
+    size_t fsmem = 0, ssmem = 0, fsmem_small = 0, ssmem_small = 0, fsmem_large = 0, ssmem_large = 0;
+    const size_t limit = nd_large_limit(smem_optin);
     for (int s = 0; s < nsteps; ++s) {
         plan[s] = nd_level_plan(sym, s, mb, fsz, cta_warps_f, cta_threads_s);
         plan_small[s] = plan[s].small;
         if (plan[s].small) { fsmem_small = std::max(fsmem_small, plan[s].smem_f); ssmem_small = std::max(ssmem_small, plan[s].smem_s); }
         // every level can also run on the generic kernels
-        fsmem = std::max(fsmem, nd_factor_smem(plan[s].nFw, s > 0 ? mb * sym.step_max_ring_pix[s - 1] : 0));
-        ssmem = std::max(ssmem, nd_solve_smem(plan[s].nFw));
+        if (!nd_level_large(plan[s], limit, smem_optin, large)) return -1;
+        size_t &f = plan[s].large_f ? fsmem_large : fsmem, &g = plan[s].large_s ? ssmem_large : ssmem;
+        f = std::max(f, nd_level_smem_f(plan[s]));
+        g = std::max(g, nd_level_smem_s(plan[s]));
     }
-    return nd_kernel_attributes(w, fsmem, ssmem, fsmem_small, ssmem_small, smem_optin);
+    return nd_kernel_attributes(w, fsmem, ssmem, fsmem_small, ssmem_small, smem_optin, 0, fsmem_large, ssmem_large);
+}
+
+using NdFactorKernel = void (*)(NdDev, int, int, double, int);
+// the generic factorisation kernel of a level: block width, where the panel lives, alone or shared by a cluster
+static NdFactorKernel nd_factor_kernel_of(const NdLevelPlan &lp, bool cluster)
+{
+    if (lp.large_f)
+        return lp.nb != ND_NB ? (cluster ? nd_factor8_large_cluster_kernel : nd_factor8_large_kernel)
+                              : (cluster ? nd_factor_large_cluster_kernel : nd_factor_large_kernel);
+    return lp.nb != ND_NB ? (cluster ? nd_factor8_cluster_kernel : nd_factor8_kernel) : (cluster ? nd_factor_cluster_kernel : nd_factor_kernel);
 }
 
 // CTAs per front of a level (a thread-block cluster shares the front: nd_factor_body<true>): the top levels of the tree
@@ -237,15 +295,15 @@ static int nd_cluster_size(const NdLevelPlan &lp, int cnt, int sm_count)
     return (int)std::max<long long>(1, C);
 }
 
-// how many clusters of C CTAs (threads, dynamic shared memory) the device runs at once: asked of the driver once per shape
-static int nd_active_clusters(int C, int threads, size_t smem, int nb = ND_NB)
+// how many clusters of C CTAs (threads, dynamic shared memory) of kernel k the device runs at once: asked of the driver
+// once per shape
+static int nd_active_clusters(NdFactorKernel k, int C, int threads, size_t smem)
 {
     static std::mutex mu;
-    static std::unordered_map<unsigned long long, int> memo;
+    static std::map<std::tuple<int, int, int, size_t, NdFactorKernel>, int> memo;
     int dev = 0;
     cudaGetDevice(&dev);
-    const unsigned long long key = ((unsigned long long)dev << 48) ^ ((unsigned long long)C << 40) ^ ((unsigned long long)threads << 24) ^
-                                   ((unsigned long long)(nb == ND_NB ? 0 : 1) << 63) ^ (unsigned long long)(smem >> 8);
+    const auto key = std::make_tuple(dev, C, threads, smem, k);
     std::lock_guard<std::mutex> lock(mu);
     auto it = memo.find(key);
     if (it != memo.end()) return it->second;
@@ -256,8 +314,7 @@ static int nd_active_clusters(int C, int threads, size_t smem, int nb = ND_NB)
     attr[0].val.clusterDim.x = (unsigned)C; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
     int nclusters = 0;
-    const cudaError_t qe = nb == ND_NB ? cudaOccupancyMaxActiveClusters(&nclusters, nd_factor_cluster_kernel, &cfg)
-                                       : cudaOccupancyMaxActiveClusters(&nclusters, nd_factor8_cluster_kernel, &cfg);
+    const cudaError_t qe = cudaOccupancyMaxActiveClusters(&nclusters, k, &cfg);
     if (qe != cudaSuccess) { cudaGetLastError(); nclusters = 0; }
     memo[key] = nclusters;
     return nclusters;
@@ -266,9 +323,10 @@ static int nd_active_clusters(int C, int threads, size_t smem, int nb = ND_NB)
 // launch of the cluster-shared front factorisation; the cluster shrinks until the device runs all fronts of the level at once
 static cudaError_t nd_launch_factor_cluster(const NdDev &nd, const NdLevelPlan &lp, int s, int cnt, int C, double guard, cudaStream_t st)
 {
-    const size_t smem = nd_factor_smem(lp.nFw, lp.nRc, lp.nb);
+    const size_t smem = nd_level_smem_f(lp);
     const long long fronts = (long long)lp.nfr * cnt;
-    while (C > 1 && nd_active_clusters(C, lp.threads_f, smem, lp.nb) < fronts) --C;
+    const NdFactorKernel kc = nd_factor_kernel_of(lp, true);
+    while (C > 1 && nd_active_clusters(kc, C, lp.threads_f, smem) < fronts) --C;
     if (C > 1) {
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3((unsigned)(lp.nfr * C), (unsigned)cnt);
@@ -279,12 +337,32 @@ static cudaError_t nd_launch_factor_cluster(const NdDev &nd, const NdLevelPlan &
         attr[0].id = cudaLaunchAttributeClusterDimension;
         attr[0].val.clusterDim.x = (unsigned)C; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
         cfg.attrs = attr; cfg.numAttrs = 1;
-        if (lp.nb != ND_NB) return cudaLaunchKernelEx(&cfg, nd_factor8_cluster_kernel, nd, lp.t0, s & 1, guard, lp.nFw);
-        return cudaLaunchKernelEx(&cfg, nd_factor_cluster_kernel, nd, lp.t0, s & 1, guard, lp.nFw);
+        return cudaLaunchKernelEx(&cfg, kc, nd, lp.t0, s & 1, guard, lp.nFw);
     }
-    if (lp.nb != ND_NB) nd_factor8_kernel<<<dim3(lp.nfr, cnt), lp.threads_f, smem, st>>>(nd, lp.t0, s & 1, guard, lp.nFw);
-    else nd_factor_kernel<<<dim3(lp.nfr, cnt), lp.threads_f, smem, st>>>(nd, lp.t0, s & 1, guard, lp.nFw);
+    nd_factor_kernel_of(lp, false)<<<dim3(lp.nfr, cnt), lp.threads_f, smem, st>>>(nd, lp.t0, s & 1, guard, lp.nFw);
     return cudaGetLastError();
+}
+
+// scratch of the large-front variants (doubles per image): enough for any wave, whose clusters are at most as large as
+// those of a single image
+static size_t nd_scratch_doubles(const std::vector<NdLevelPlan> &plan, int sm_count)
+{
+    size_t m = 0;
+    for (NdLevelPlan lp : plan) {
+        lp.small = false;
+        m = std::max(m, nd_level_scratch(lp, nd_cluster_size(lp, 1, sm_count)));
+    }
+    return nd_even((long long)m);
+}
+
+// the workspace could not be allocated: what one image needs, for the message
+static int nd_alloc_fail(NdWork &w, const char *what, size_t bytes, size_t per_image, cudaError_t e)
+{
+    char buf[256];
+    snprintf(buf, sizeof buf, "nested-dissection workspace (%s): %.3g GB could not be allocated, %.3g GB per image: %s", what,
+             bytes * 1e-9, per_image * 1e-9, cudaGetErrorString(e));
+    w.slots_key_n = -1;      // memory got tighter since the wave size was decided: ask again next time
+    return nd_fail(w, -6, buf);
 }
 
 // CTA width of the generic front factorisation of one level.  A level with several fronts per SM runs narrow CTAs (4
@@ -315,9 +393,9 @@ static void nd_launch_factor(const NdDev &nd, std::vector<NdLevelPlan> &plan, co
         else {
             const int C = nd_cluster_size(lp, cnt, sm_count);
             if (C > 1) nd_launch_factor_cluster(nd, lp, s, cnt, C, guard, st);
-            else if (lp.nb != ND_NB)
-                nd_factor8_kernel<<<dim3(lp.nfr, cnt), nd_factor_cta_threads(lp, cnt, sm_count), nd_factor_smem(lp.nFw, lp.nRc, lp.nb), st>>>(nd, lp.t0, s & 1, guard, lp.nFw);
-            else nd_factor_kernel<<<dim3(lp.nfr, cnt), nd_factor_cta_threads(lp, cnt, sm_count), nd_factor_smem(lp.nFw, lp.nRc), st>>>(nd, lp.t0, s & 1, guard, lp.nFw);
+            else
+                nd_factor_kernel_of(lp, false)<<<dim3(lp.nfr, cnt), nd_factor_cta_threads(lp, cnt, sm_count), nd_level_smem_f(lp), st>>>(
+                    nd, lp.t0, s & 1, guard, lp.nFw);
         }
     }
     *launches += nsteps;
@@ -333,6 +411,8 @@ static void nd_launch_solve(const NdDev &nd, const std::vector<NdLevelPlan> &pla
         if (lp.small)
             nd_fwd_small_kernel<<<dim3((lp.nfr + ND_SMALL_WARPS - 1) / ND_SMALL_WARPS, cnt), 32 * ND_SMALL_WARPS, lp.smem_s, st>>>(
                 nd, lp.t0, lp.nfr, s & 1, vec, stride, lp.arena_s);
+        else if (lp.large_s)
+            nd_fwd_large_kernel<<<dim3(lp.nfr, cnt), lp.threads_s, nd_level_smem_s(lp), st>>>(nd, lp.t0, s & 1, vec, stride, lp.nFw);
         else
             nd_fwd_kernel<<<dim3(lp.nfr, cnt), lp.threads_s, nd_solve_smem(lp.nFw), st>>>(nd, lp.t0, s & 1, vec, stride);
     }
@@ -341,6 +421,8 @@ static void nd_launch_solve(const NdDev &nd, const std::vector<NdLevelPlan> &pla
         if (lp.small)
             nd_bwd_small_kernel<<<dim3((lp.nfr + ND_SMALL_WARPS - 1) / ND_SMALL_WARPS, cnt), 32 * ND_SMALL_WARPS, lp.smem_s, st>>>(
                 nd, lp.t0, lp.nfr, vec, stride, lp.arena_s);
+        else if (lp.large_s)
+            nd_bwd_large_kernel<<<dim3(lp.nfr, cnt), lp.threads_s, nd_level_smem_s(lp), st>>>(nd, lp.t0, vec, stride, lp.nFw);
         else
             nd_bwd_kernel<<<dim3(lp.nfr, cnt), lp.threads_s, nd_solve_smem(lp.nFw), st>>>(nd, lp.t0, vec, stride);
     }
@@ -352,6 +434,7 @@ static int run_gradient_nd(NdWork &w, const NdProblem &gp, int sm_count, size_t 
                            cudaStream_t st, double *d_grad_out, long long *launches)
 {
     NdWork &gw = w;
+    smem_optin = nd_dynamic_optin(smem_optin);
     const Real *gp_u = static_cast<const Real *>(gp.u), *gp_ubar = static_cast<const Real *>(gp.ubar),
                *gp_amap = static_cast<const Real *>(gp.alpha_map);
     const int n = gp.M, N = gp.M * gp.N, ng = gp.lm * gp.ln;
@@ -371,9 +454,10 @@ static int run_gradient_nd(NdWork &w, const NdProblem &gp, int sm_count, size_t 
     std::vector<NdLevelPlan> plan;
     std::vector<char> plan_small;
     {
-        const int rc = nd_prepare_levels(w, sym, mb, fsz, gp.O, smem_optin, plan, plan_small);
+        const int rc = nd_prepare_levels(w, sym, mb, fsz, gp.O, smem_optin, gp.large_fronts, plan, plan_small);
         if (rc != 0) return rc;
     }
+    const size_t scr_stride = nd_scratch_doubles(plan, sm_count);
 
     // ---- per-slot sizes.  Pools of the MULT form are estimated at 2.2× the one-unknown-per-pixel sizes (≈ 1.5
     // unknowns per pixel) and grown when a wave needs more.
@@ -381,7 +465,7 @@ static int run_gradient_nd(NdWork &w, const NdProblem &gp, int sm_count, size_t 
     const double est = node ? 1.0 : 2.2;
     const size_t fix_bytes = (size_t)NDTV_PLANES * N * 8 + (size_t)5 * mb * mb * N * 8 +
                              (node ? 0 : ((size_t)N + 2) * 4 + (size_t)6 * N * 8 + w.plan.posg_len * 4 + (size_t)4 * nf * 8 + 32) + 16;
-    const size_t pool_bytes = (size_t)(est * (double)(t1[0] + 2 * t1[1] + 2 * t1[2])) * 8;
+    const size_t pool_bytes = (size_t)(est * (double)(t1[0] + 2 * t1[1] + 2 * t1[2])) * 8 + scr_stride * 8;
     const size_t per_slot = fix_bytes + pool_bytes;
     w.last_bytes_per_image = per_slot;
     int slots = std::min(gp.O, 256);      // 256 images already give every level thousands of fronts
@@ -397,12 +481,8 @@ static int run_gradient_nd(NdWork &w, const NdProblem &gp, int sm_count, size_t 
         w.slots_key_n = n; w.slots_key_node = (int)node; w.slots_key_want = want; w.slots_cached = slots;
     }
     auto need = [&](NdBuf &b, size_t bytes, const char *what) -> int {
-        cudaError_t e = b.ensure(bytes);
-        if (e != cudaSuccess) {
-            w.slots_key_n = -1;      // memory got tighter since the wave size was decided: ask again next time
-            return nd_fail(gw, -6, std::string("nested-dissection workspace (") + what + "): " + cudaGetErrorString(e));
-        }
-        return 0;
+        const cudaError_t e = b.ensure(bytes);
+        return e == cudaSuccess ? 0 : nd_alloc_fail(gw, what, bytes, w.last_bytes_per_image, e);
     };
     int rc = 0;
     NdTvSlots ws;
@@ -478,15 +558,18 @@ static int run_gradient_nd(NdWork &w, const NdProblem &gp, int sm_count, size_t 
             Ls = (size_t)m[0]; Us = (size_t)m[1]; UVs = (size_t)m[2];
         }
         Ls = (Ls + 1) & ~(size_t)1; Us = (Us + 1) & ~(size_t)1; UVs = (UVs + 1) & ~(size_t)1;
+        w.last_bytes_per_image = fix_bytes + (Ls + 2 * Us + 2 * UVs + scr_stride) * 8;
         if ((rc = need(w.L, Ls * 8 * cnt, "factors"))) return rc;
         if ((rc = need(w.U0, Us * 8 * cnt, "update matrices"))) return rc;
         if ((rc = need(w.U1, Us * 8 * cnt, "update matrices"))) return rc;
         if ((rc = need(w.UV0, UVs * 8 * cnt, "update vectors"))) return rc;
         if ((rc = need(w.UV1, UVs * 8 * cnt, "update vectors"))) return rc;
+        if (scr_stride && (rc = need(w.scr, scr_stride * 8 * cnt, "large-front scratch"))) return rc;
         nd.L = (double *)w.L.p; nd.L_stride = Ls;
         nd.U[0] = (double *)w.U0.p; nd.U[1] = (double *)w.U1.p; nd.U_stride = Us;
         nd.UV[0] = (double *)w.UV0.p; nd.UV[1] = (double *)w.UV1.p; nd.UV_stride = UVs;
-        w.last_bytes_per_image = fix_bytes + (Ls + 2 * Us + 2 * UVs) * 8;
+        nd.scr = (double *)w.scr.p; nd.scr_stride = scr_stride;
+        w.last_bytes_per_image = fix_bytes + (Ls + 2 * Us + 2 * UVs + scr_stride) * 8;
 
         nd_launch_factor(nd, plan, plan_small, sym, mb, cnt, sm_count, guard, st, launches);
         auto solve = [&](double *vec, size_t stride) { nd_launch_solve(nd, plan, cnt, vec, stride, st, launches); };
@@ -532,6 +615,7 @@ static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, s
 {
     const Real *gp_u = static_cast<const Real *>(gp.u), *gp_ubar = static_cast<const Real *>(gp.ubar);
     const int n = gp.M, N = gp.M * gp.N, nops = 3, ng = 1;
+    smem_optin = nd_dynamic_optin(smem_optin);
     if (gp.M != gp.N) return nd_fail(w, -1, "square images required");
     if (n < 8) return -1;                                   // tiny images: the band LU
     {
@@ -544,13 +628,14 @@ static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, s
     std::vector<NdLevelPlan> plan;
     std::vector<char> plan_small;
     {
-        const int rc = nd_prepare_levels(w, sym, 1, 1.0, gp.O, smem_optin, plan, plan_small);
+        const int rc = nd_prepare_levels(w, sym, 1, 1.0, gp.O, smem_optin, gp.large_fronts, plan, plan_small);
         if (rc != 0) return rc;
     }
     const long long *t1 = w.plan.tot1;
     const size_t pix_stride = (size_t)LU_PLANES * N, ast_stride = (size_t)ND3_NH * N;
     const size_t Ls = ((size_t)t1[0] + 1) & ~(size_t)1, Us = ((size_t)t1[1] + 1) & ~(size_t)1, UVs = ((size_t)t1[2] + 1) & ~(size_t)1;
-    const size_t per_slot = (pix_stride + ast_stride + Ls + 2 * Us + 2 * UVs) * 8 + 16;
+    const size_t scr_stride = nd_scratch_doubles(plan, sm_count);
+    const size_t per_slot = (pix_stride + ast_stride + Ls + 2 * Us + 2 * UVs + scr_stride) * 8 + 16;
     w.last_bytes_per_image = per_slot;
     int slots = std::min(gp.O, 256);
     if (w.slots_key_n == n && w.slots_key_node == 3 && w.slots_key_want == slots) {
@@ -565,12 +650,8 @@ static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, s
         w.slots_key_n = n; w.slots_key_node = 3; w.slots_key_want = want; w.slots_cached = slots;
     }
     auto need = [&](NdBuf &b, size_t bytes, const char *what) -> int {
-        cudaError_t e = b.ensure(bytes);
-        if (e != cudaSuccess) {
-            w.slots_key_n = -1;
-            return nd_fail(w, -6, std::string("nested-dissection workspace (") + what + "): " + cudaGetErrorString(e));
-        }
-        return 0;
+        const cudaError_t e = b.ensure(bytes);
+        return e == cudaSuccess ? 0 : nd_alloc_fail(w, what, bytes, w.last_bytes_per_image, e);
     };
     int rc = 0;
     if ((rc = need(w.pix, pix_stride * 8 * slots, "pixel planes"))) return rc;
@@ -584,6 +665,7 @@ static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, s
     if ((rc = need(w.U1, Us * 8 * slots, "update matrices"))) return rc;
     if ((rc = need(w.UV0, UVs * 8 * slots, "update vectors"))) return rc;
     if ((rc = need(w.UV1, UVs * 8 * slots, "update vectors"))) return rc;
+    if (scr_stride && (rc = need(w.scr, scr_stride * 8 * slots, "large-front scratch"))) return rc;
 
     LuSlots ws;
     ws.ab = nullptr; ws.ab_stride = 0; ws.pix = (double *)w.pix.p; ws.pix_stride = pix_stride; ws.info = (int *)w.info.p;
@@ -606,6 +688,7 @@ static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, s
     nd.UV[0] = (double *)w.UV0.p; nd.UV[1] = (double *)w.UV1.p; nd.UV_stride = UVs;
     nd.ast = (const double *)w.ast.p; nd.ast_stride = ast_stride;
     nd.info = (int *)w.info.p;
+    nd.scr = (double *)w.scr.p; nd.scr_stride = scr_stride;
 
     const double tol = gp.tol > 0 ? gp.tol : 1e300;
     const int refine = gp.maxit > 0 ? std::min(gp.maxit, 8) : 1;
@@ -640,7 +723,8 @@ static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, s
 // ---------------------------------------------------------------------------
 // sumregs_gradient (non-regularised) on the same solver: multiplier space, 3-6 unknowns per pixel, W = 2.  Front sizes
 // are data: measured per level on the device (nd_level_sizes_kernel) and read back with the pool totals, one
-// synchronisation per wave; a front beyond shared memory sends the call back to the band Cholesky (-1).
+// synchronisation per wave; a front beyond shared memory sends the call back to the band Cholesky (-1), or, with
+// gp.large_fronts (the band Cholesky refused the shape too), to the large-front variants.
 // ---------------------------------------------------------------------------
 template <typename Real>
 static int run_gradient3_nd_mult(NdWork &w, const Nd3mProblem &gp, int sm_count, size_t smem_optin, cudaStream_t st,
@@ -649,6 +733,7 @@ static int run_gradient3_nd_mult(NdWork &w, const Nd3mProblem &gp, int sm_count,
     const Real *gp_u = static_cast<const Real *>(gp.u), *gp_ubar = static_cast<const Real *>(gp.ubar),
                *gp_amaps = static_cast<const Real *>(gp.alpha_maps);
     const int n = gp.M, N = gp.M * gp.N, ng = gp.lm * gp.ln, mb = ND3M_MB;
+    smem_optin = nd_dynamic_optin(smem_optin);
     if (gp.M != gp.N) return nd_fail(w, -1, "square images required");
     if (n < 8) return -1;
     if (3 * ng > 65536) return nd_fail(w, -1, "lambda grid too large");
@@ -686,12 +771,8 @@ static int run_gradient3_nd_mult(NdWork &w, const Nd3mProblem &gp, int sm_count,
         w.slots_key_n = n; w.slots_key_node = 4; w.slots_key_want = want; w.slots_cached = slots;
     }
     auto need = [&](NdBuf &b, size_t bytes, const char *what) -> int {
-        cudaError_t e = b.ensure(bytes);
-        if (e != cudaSuccess) {
-            w.slots_key_n = -1;
-            return nd_fail(w, -6, std::string("nested-dissection workspace (") + what + "): " + cudaGetErrorString(e));
-        }
-        return 0;
+        const cudaError_t e = b.ensure(bytes);
+        return e == cudaSuccess ? 0 : nd_alloc_fail(w, what, bytes, w.last_bytes_per_image, e);
     };
     int rc = 0;
     if ((rc = need(w.out_img, (size_t)gp.O * 3 * ng * 8, "per-image gradients"))) return rc;
@@ -762,30 +843,39 @@ static int run_gradient3_nd_mult(NdWork &w, const Nd3mProblem &gp, int sm_count,
             w.slots_cached = slots;
             continue;
         }
-        size_t fsmem = 0, fsmem8 = 0, ssmem = 0;
+        size_t fsmem = 0, fsmem8 = 0, ssmem = 0, fsmem_large = 0, ssmem_large = 0;
         // test hook: BPLTV_ND3_SMEM_KB lowers the shared memory the 16-column panel may take (sends fronts to the 8-column kernels)
         const char *skb = bpltv::env_get("BPLTV_ND3_SMEM_KB");
         const size_t smem_plan = skb && *skb ? std::min<size_t>(smem_optin, (size_t)atoi(skb) << 10) : smem_optin;
+        const size_t limit = nd_large_limit(smem_optin);
         for (int s = 0; s < nsteps; ++s) {
             plan[s] = nd_level_plan_sized(sym, s, h_lvl[2 * s], s > 0 ? h_lvl[2 * (s - 1) + 1] : 0, smem_plan, cta_warps_f, 512);
-            if (plan[s].nb == ND_NB) fsmem = std::max(fsmem, plan[s].smem_f); else fsmem8 = std::max(fsmem8, plan[s].smem_f);
-            ssmem = std::max(ssmem, plan[s].smem_s);
+            if (!nd_level_large(plan[s], limit, smem_optin, gp.large_fronts)) return -1;      // the band Cholesky first
+            if (plan[s].large_f) fsmem_large = std::max(fsmem_large, plan[s].smem_f);
+            else if (plan[s].nb == ND_NB) fsmem = std::max(fsmem, plan[s].smem_f);
+            else fsmem8 = std::max(fsmem8, plan[s].smem_f);
+            size_t &g = plan[s].large_s ? ssmem_large : ssmem;
+            g = std::max(g, plan[s].smem_s);
         }
+        const size_t scr_stride = nd_scratch_doubles(plan, sm_count);
+        w.last_bytes_per_image += scr_stride * 8;
         {   // test hook: BPLTV_ND3_MAXF caps the front size this path takes (exercises the fall-back below)
             const char *mf = bpltv::env_get("BPLTV_ND3_MAXF");
             if (mf && *mf)
                 for (int s = 0; s < nsteps; ++s)
                     if (h_lvl[2 * s] > atoi(mf)) return -1;
         }
-        if ((rc = nd_kernel_attributes(w, fsmem, ssmem, 0, 0, smem_optin, fsmem8))) return rc;      // -1: the band Cholesky
+        if ((rc = nd_kernel_attributes(w, fsmem, ssmem, 0, 0, smem_optin, fsmem8, fsmem_large, ssmem_large))) return rc;
         if ((rc = need(w.L, Ls * 8 * cnt, "factors"))) return rc;
         if ((rc = need(w.U0, Us * 8 * cnt, "update matrices"))) return rc;
         if ((rc = need(w.U1, Us * 8 * cnt, "update matrices"))) return rc;
         if ((rc = need(w.UV0, UVs * 8 * cnt, "update vectors"))) return rc;
         if ((rc = need(w.UV1, UVs * 8 * cnt, "update vectors"))) return rc;
+        if (scr_stride && (rc = need(w.scr, scr_stride * 8 * cnt, "large-front scratch"))) return rc;
         nd.L = (double *)w.L.p; nd.L_stride = Ls;
         nd.U[0] = (double *)w.U0.p; nd.U[1] = (double *)w.U1.p; nd.U_stride = Us;
         nd.UV[0] = (double *)w.UV0.p; nd.UV[1] = (double *)w.UV1.p; nd.UV_stride = UVs;
+        nd.scr = (double *)w.scr.p; nd.scr_stride = scr_stride;
 
         nd_launch_factor(nd, plan, plan_small, sym, mb, cnt, sm_count, guard, st, launches);
         double *zeta = ws.vec + (size_t)mb * N, *work = ws.vec + (size_t)2 * mb * N;

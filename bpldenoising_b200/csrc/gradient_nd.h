@@ -21,6 +21,7 @@ struct NdProblem {
     double gamma, act_tol, eps_act;
     double tol;                 // backward error above which the result is poisoned with NaN (≤ 0: never)
     int maxit;                  // refinement steps (≤ 0: default)
+    bool large_fronts;          // fronts beyond shared memory take the large-front variants instead of returning -1
 };
 
 // scalar sumregs_gradient_reg of /root/reference/src/SumRegsLearningFunction.jl:112-167 (three difference operators,
@@ -33,6 +34,7 @@ struct Nd3Problem {
     double gamma;
     double tol;                 // backward error above which the result is poisoned with NaN (≤ 0: never)
     int maxit;                  // refinement steps (≤ 0: default)
+    bool large_fronts;          // fronts beyond shared memory take the large-front variants instead of returning -1
 };
 
 // sumregs_gradient (non-regularised; scalar :264-327, patch :330-407) in multiplier space: 3-6 unknowns per pixel,
@@ -46,6 +48,7 @@ struct Nd3mProblem {
     double act_tol, eps_act;
     double tol;                 // relative residual above which the result is poisoned with NaN (≤ 0: never)
     int maxit;                  // refinement steps (≤ 0: default)
+    bool large_fronts;          // fronts beyond shared memory take the large-front variants instead of returning -1
 };
 
 NdWork *nd_work_create();
@@ -53,7 +56,8 @@ void nd_work_destroy(NdWork *w);
 const char *nd_work_error(const NdWork *w);
 size_t nd_work_bytes_per_image(const NdWork *w);
 const double *nd_work_relres_max(const NdWork *w);      // device pointer: worst backward error of the last call
-// 0 ok; -1: the shape is not taken (fronts beyond shared memory) — use the band solver; other negatives: bpltv_status
+// 0 ok; -1: the shape is not taken (fronts beyond shared memory and large_fronts not set) — use the band solver; other
+// negatives: bpltv_status (BPLTV_ERR_ALLOC: the workspace of one image does not fit; the message names its size)
 int nd_run_gradient(NdWork *w, const NdProblem &gp, int sm_count, size_t smem_optin, cudaStream_t st, double *d_grad_out,
                     long long *launches);
 // d_grad_out: 3 doubles (one per operator).  Use a workspace of its own (the plan is keyed by the coupling radius).

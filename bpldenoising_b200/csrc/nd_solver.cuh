@@ -54,6 +54,8 @@ struct NdDev {
     double *UV[2]; size_t UV_stride;
     const double *ast; size_t ast_stride;
     int *info;                            // per slot: [0] pivots raised (floor / bound), [1] ≠ 0: the factorisation broke down
+    double *scr = nullptr;                // per slot: scratch of the large-front variants (nd_level_scratch)
+    size_t scr_stride = 0;
 };
 
 #ifdef BPLTV_EMU
@@ -263,11 +265,12 @@ static __device__ __forceinline__ double *nd_col(double *L, double *U, int nP, i
 }
 
 static __host__ __device__ __forceinline__ int nd_panel_pitch(int nFmax) { return (nFmax + 31) & ~31; }
-// dynamic shared memory of nd_factor_kernel (bytes): S0, S, reciprocal diagonal, column floors, panel P (NB × pitch),
-// the child map (ints)
-static inline size_t nd_factor_smem(int nFmax, int nRchild_max, int nb = ND_NB)
+// dynamic shared memory of nd_factor_kernel (bytes): S0, S, reciprocal diagonal, column floors, panel P (NB × pitch;
+// not on the large-front variants, which keep it in global memory), the child map (ints)
+static inline size_t nd_factor_smem(int nFmax, int nRchild_max, int nb = ND_NB, bool panel_global = false)
 {
-    return (size_t)(2 * nb * nb + 2 * nb + nb * nd_panel_pitch(nFmax)) * sizeof(double) + (((size_t)nRchild_max * sizeof(int) + 15) & ~(size_t)15);
+    return (size_t)(2 * nb * nb + 2 * nb + (panel_global ? 0 : nb * nd_panel_pitch(nFmax))) * sizeof(double) +
+           (((size_t)nRchild_max * sizeof(int) + 15) & ~(size_t)15);
 }
 
 // ---------------------------------------------------------------------------
@@ -281,15 +284,19 @@ static inline size_t nd_factor_smem(int nFmax, int nRchild_max, int nb = ND_NB)
 // NB: columns per block step.  16 everywhere, except for fronts whose 16-column panel exceeds shared memory (the
 // sum-of-regularisers multiplier form of a large or mostly flat image: > ≈ 1700 unknowns), which take 8 — twice the steps
 // for half the panel.  (The factor does not depend on NB beyond the order of the updates; the solves use blocks of 16.)
-template <bool CL, int NB>
+// PG (large fronts, whose panel does not fit in shared memory even at 8 columns): the panel lives in global memory, in
+// the CTA's own slice of nd.scr (NB × pitch doubles at blockIdx.x; a cluster's CTAs each form their own copy, as in
+// shared memory).  Nothing else changes: the same operations in the same order, the same bits.
+template <bool CL, int NB, bool PG = false>
 static __device__ __forceinline__ void nd_factor_body(const NdDev &nd, int t0, int par, double guard, int nFmax)
 {
     ND_DYN_SMEM(sm);
-    double *S0 = sm, *S = sm + NB * NB, *dinv = sm + 2 * NB * NB, *dfl = dinv + NB, *P = dfl + NB;
+    const int PR = nd_panel_pitch(nFmax);
+    double *S0 = sm, *S = sm + NB * NB, *dinv = sm + 2 * NB * NB, *dfl = dinv + NB;
+    double *P = PG ? nd.scr + nd.scr_stride * blockIdx.y + (size_t)blockIdx.x * NB * PR : dfl + NB;
     __shared__ int s_cbad;
     __shared__ unsigned long long s_amax2;
-    const int PR = nd_panel_pitch(nFmax);
-    int *umap = reinterpret_cast<int *>(P + (size_t)NB * PR);
+    int *umap = reinterpret_cast<int *>(PG ? dfl + NB : P + (size_t)NB * PR);
     const int tid = threadIdx.x, T = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarps = T >> 5;
     int crank = 0, csize = 1;
     if (CL) {
@@ -516,10 +523,20 @@ __global__ void __launch_bounds__(512) nd_factor_cluster_kernel(NdDev nd, int t0
 // the same with 8-column block steps (fronts whose 16-column panel does not fit in shared memory)
 __global__ void __launch_bounds__(512) nd_factor8_kernel(NdDev nd, int t0, int par, double guard, int nFmax) { nd_factor_body<false, 8>(nd, t0, par, guard, nFmax); }
 __global__ void __launch_bounds__(512) nd_factor8_cluster_kernel(NdDev nd, int t0, int par, double guard, int nFmax) { nd_factor_body<true, 8>(nd, t0, par, guard, nFmax); }
+// large fronts: the panel in global memory (nd.scr).  16-column block steps for fronts beyond the 8-column panel, and for
+// levels sent here by BPLTV_ND_LARGE_KB, the block width their shared-memory kernel would have used
+__global__ void __launch_bounds__(512) nd_factor_large_kernel(NdDev nd, int t0, int par, double guard, int nFmax) { nd_factor_body<false, ND_NB, true>(nd, t0, par, guard, nFmax); }
+__global__ void __launch_bounds__(512) nd_factor_large_cluster_kernel(NdDev nd, int t0, int par, double guard, int nFmax) { nd_factor_body<true, ND_NB, true>(nd, t0, par, guard, nFmax); }
+__global__ void __launch_bounds__(512) nd_factor8_large_kernel(NdDev nd, int t0, int par, double guard, int nFmax) { nd_factor_body<false, 8, true>(nd, t0, par, guard, nFmax); }
+__global__ void __launch_bounds__(512) nd_factor8_large_cluster_kernel(NdDev nd, int t0, int par, double guard, int nFmax) { nd_factor_body<true, 8, true>(nd, t0, par, guard, nFmax); }
 
-// dynamic shared memory of the solve kernels (bytes): the front's vector, the ring sums of the backward sweep, two
-// diagonal blocks (the next one is fetched while the current one is used), NB scratch
-static inline size_t nd_solve_smem(int nFmax) { return (size_t)(2 * ((nFmax + 1) & ~1) + 2 * ND_NB * ND_NB + 2 * ND_NB + 2) * sizeof(double); }
+// dynamic shared memory of the solve kernels (bytes): the front's vector, the ring sums of the backward sweep (both in
+// global memory on the large-front variants), two diagonal blocks (the next one is fetched while the current one is
+// used), NB scratch
+static inline size_t nd_solve_smem(int nFmax, bool vec_global = false)
+{
+    return (size_t)((vec_global ? 0 : 2 * ((nFmax + 1) & ~1)) + 2 * ND_NB * ND_NB + 2 * ND_NB + 2) * sizeof(double);
+}
 
 // diagonal block kb of the factor → registers (≤ 4 per thread, CTAs of ≥ 64 threads) → shared memory, so that the global
 // latency of the NEXT block hides behind the substitution of the current one
@@ -552,8 +569,11 @@ static __device__ __forceinline__ void nd_diag_store(double *S, int tid, int T, 
 // Only the PIVOT rows are updated inside the serial block loop; the ring rows (the bulk of a front) take all their
 // blocks in one parallel pass afterwards, block by block in the same order — the same sums, the same bits as a loop that
 // updates every row at every step, with a chain of nP/16 short steps instead of nP/16 passes over the whole front.
+// VG (large fronts): the front's vector lives in global memory, in the front's slice of nd.scr (2·even(nFmax) doubles at
+// blockIdx.x); the same sums in the same order.
 // ---------------------------------------------------------------------------
-__global__ void nd_fwd_kernel(NdDev nd, int t0, int par, double *vec_all, size_t vec_stride)
+template <bool VG>
+static __device__ __forceinline__ void nd_fwd_body(const NdDev &nd, int t0, int par, double *vec_all, size_t vec_stride, int nFmax)
 {
     ND_DYN_SMEM(sm);
     constexpr int NB = ND_NB;
@@ -568,7 +588,8 @@ __global__ void nd_fwd_kernel(NdDev nd, int t0, int par, double *vec_all, size_t
     double *uv = nd.UV[par] + nd.UV_stride * slot + foff[4 * (size_t)t + 2];
     double *vec = vec_all + vec_stride * slot;
     const int nFe = (nF + 1) & ~1;
-    double *v = sm, *Sb = sm + 2 * nFe, *ys = Sb + 2 * NB * NB;
+    double *v = VG ? nd.scr + nd.scr_stride * slot + (size_t)blockIdx.x * 2 * nd_even(nFmax) : sm;
+    double *Sb = VG ? sm : sm + 2 * nFe, *ys = Sb + 2 * NB * NB;
     double sreg[4];
 
     if (nP > 0) nd_diag_fetch(L, nF, nP, 0, tid, T, sreg);
@@ -664,13 +685,16 @@ __global__ void nd_fwd_kernel(NdDev nd, int t0, int par, double *vec_all, size_t
     }
     for (int r = tid; r < nR; r += T) uv[r] = v[nP + r];
 }
+__global__ void nd_fwd_kernel(NdDev nd, int t0, int par, double *vec_all, size_t vec_stride) { nd_fwd_body<false>(nd, t0, par, vec_all, vec_stride, 0); }
+__global__ void nd_fwd_large_kernel(NdDev nd, int t0, int par, double *vec_all, size_t vec_stride, int nFmax) { nd_fwd_body<true>(nd, t0, par, vec_all, vec_stride, nFmax); }
 
 // ---------------------------------------------------------------------------
 // backward substitution, one level: x_P = L11⁻ᵀ(y_P − L21ᵀ x_ring); the ring's x comes from the ancestors.
 // The ring part of every pivot column's dot product is formed up front, in parallel (a warp per column); the serial
-// block loop adds the part over the pivot rows below the block.
+// block loop adds the part over the pivot rows below the block.  VG: as nd_fwd_body.
 // ---------------------------------------------------------------------------
-__global__ void nd_bwd_kernel(NdDev nd, int t0, double *vec_all, size_t vec_stride)
+template <bool VG>
+static __device__ __forceinline__ void nd_bwd_body(const NdDev &nd, int t0, double *vec_all, size_t vec_stride, int nFmax)
 {
     ND_DYN_SMEM(sm);
     constexpr int NB = ND_NB;
@@ -684,7 +708,8 @@ __global__ void nd_bwd_kernel(NdDev nd, int t0, double *vec_all, size_t vec_stri
     const double *L = nd.L + nd.L_stride * slot + foff[4 * (size_t)t];
     double *vec = vec_all + vec_stride * slot;
     const int nFe = (nF + 1) & ~1;
-    double *v = sm, *tR = sm + nFe, *Sb = sm + 2 * nFe, *ts = Sb + 2 * NB * NB;
+    double *v = VG ? nd.scr + nd.scr_stride * slot + (size_t)blockIdx.x * 2 * nd_even(nFmax) : sm, *tR = v + nFe;
+    double *Sb = VG ? sm : sm + 2 * nFe, *ts = Sb + 2 * NB * NB;
     double sreg[4];
     const int nblk = (nP + NB - 1) / NB;
 
@@ -751,6 +776,8 @@ __global__ void nd_bwd_kernel(NdDev nd, int t0, double *vec_all, size_t vec_stri
         for (int al = 0; al < m; ++al) vec[g0 + al] = v[a0 + al];
     }
 }
+__global__ void nd_bwd_kernel(NdDev nd, int t0, double *vec_all, size_t vec_stride) { nd_bwd_body<false>(nd, t0, vec_all, vec_stride, 0); }
+__global__ void nd_bwd_large_kernel(NdDev nd, int t0, double *vec_all, size_t vec_stride, int nFmax) { nd_bwd_body<true>(nd, t0, vec_all, vec_stride, nFmax); }
 
 
 // ===========================================================================
@@ -1088,6 +1115,8 @@ struct NdLevelPlan {
     int threads_f, threads_s;   // generic kernels: CTA sizes of the factorisation / of the solves
     size_t smem_f, smem_s;      // dynamic shared memory of the factorisation / of the solves
     int arena_f, arena_s;       // small kernels: arena (doubles)
+    bool large_f = false;       // generic factorisation with the panel in global memory (nd_factor_*large*)
+    bool large_s = false;       // generic solves with the front vector in global memory (nd_fwd/bwd_large_kernel)
 };
 static inline NdLevelPlan nd_level_plan(const NdSymbolic &sym, int s, int mb, double typ_per_pixel, int max_warps_f = 16,
                                        int max_threads_s = 512)
@@ -1134,6 +1163,35 @@ static inline NdLevelPlan nd_level_plan_sized(const NdSymbolic &sym, int s, int 
     lp.smem_f = nd_factor_smem(lp.nFw, lp.nRc, lp.nb);
     lp.smem_s = nd_solve_smem(lp.nFw);
     return lp;
+}
+
+// shared memory of the generic kernels of a level, as they will be launched
+static inline size_t nd_level_smem_f(const NdLevelPlan &lp) { return nd_factor_smem(lp.nFw, lp.nRc, lp.nb, lp.large_f); }
+static inline size_t nd_level_smem_s(const NdLevelPlan &lp) { return nd_solve_smem(lp.nFw, lp.large_s); }
+
+// Sends the generic kernels of a level to the large-front variants when their shared memory would exceed `limit` bytes
+// (the opt-in maximum, or less under a test hook).  A front beyond the 8-column panel takes 16-column block steps there
+// (half the steps, half the passes over the trailing matrix); a level sent by the hook alone keeps its block width, and
+// so its bits.  false: the level needs the variants for a front beyond `smem_optin` but `allow` is not set — the caller
+// lets a band solver try the shape first, as before the variants existed.
+static inline bool nd_level_large(NdLevelPlan &lp, size_t limit, size_t smem_optin, bool allow)
+{
+    const size_t f = nd_factor_smem(lp.nFw, lp.nRc, lp.nb), s = nd_solve_smem(lp.nFw);
+    if (!allow && (f > smem_optin || s > smem_optin)) return false;
+    lp.large_f = f > limit;
+    lp.large_s = s > limit;
+    if (lp.large_f && f > smem_optin) lp.nb = ND_NB;
+    if (!lp.small) { lp.smem_f = nd_level_smem_f(lp); lp.smem_s = nd_level_smem_s(lp); }
+    return true;
+}
+
+// scratch (doubles per image) of a level on the large-front variants with C CTAs per front: one panel per CTA, the
+// vector and the ring sums per front
+static inline size_t nd_level_scratch(const NdLevelPlan &lp, int C)
+{
+    const size_t f = lp.large_f ? (size_t)lp.nfr * C * lp.nb * nd_panel_pitch(lp.nFw) : 0;
+    const size_t s = lp.large_s ? (size_t)lp.nfr * 2 * nd_even(lp.nFw) : 0;
+    return std::max(f, s);
 }
 
 // largest front and largest ring (unknowns) of every level over the images of the wave → lvl[2s], lvl[2s+1] (zeroed by

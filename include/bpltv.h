@@ -198,7 +198,12 @@ int bpltv_sumregs_denoise(bpltv_ctx *ctx, const double *noisy, int M, int N, int
  * : sumregs_gradient_reg (:112-167), summed over images (:87-110, :169-193).  grad_out has the shape
  * of x: 3 (lm = ln = 1) or lm×ln×3 entries.  The patch variant of sumregs_gradient_reg (:195-262),
  * whose system is row-scaled by a different λ-map per operator and therefore not symmetric, is
- * solved by a banded LU in node space (γ = opts->gamma_patch).  opts == NULL → the
+ * solved by a banded LU in node space (γ = opts->gamma_patch) and is limited to M = N ≤ 430 (it
+ * would need an unsymmetric multifrontal LU).  The symmetric variants take any square size: where
+ * the fronts of the nested-dissection solver outgrow shared memory and the band solvers refuse
+ * the size too, its large-front kernels (panel and front vector in global memory) take over; an
+ * image whose workspace does not fit in device memory returns BPLTV_ERR_ALLOC, and
+ * bpltv_last_error names the gigabytes one image needs.  opts == NULL → the
  * sum-of-regularisers defaults.                                                              */
 int bpltv_sumregs_learn_eval(bpltv_ctx *ctx, const double *lam, int lm, int ln, double Delta,
                              const bpltv_eval_opts *opts, double *u_out, double *cost_out,
