@@ -1166,18 +1166,22 @@ static int run_tv_gradient(Dev &d, const GradProblem<Real> &gp, cudaStream_t st,
 // The sum-of-regularisers gradient (eval_opts.solver as above).  Scalar sumregs_gradient_reg (:112-167) is symmetric
 // positive definite in node space with coupling radius 2, and sumregs_gradient (non-regularised, scalar :264-327 and
 // patch :330-407) is the same in multiplier space (3-6 unknowns per pixel): both take the nested-dissection
-// multifrontal Cholesky.  Solver 1, the patch sumregs_gradient_reg, a shape the fronts do not take (-1) or one that
-// does not fit in memory go to the node-space band LU / compliance-form band Cholesky of run_gradient3, which needs
-// less memory per image.  A shape the band solvers refuse as well (above 430² for the band LU, 136² for the band
-// Cholesky) goes back to the fronts with their large-front variants; a failure there is final, and an image whose
-// workspace does not fit returns BPLTV_ERR_ALLOC with the size it needs.
+// multifrontal Cholesky.  Solver 1, a shape the fronts do not take (-1) or one that does not fit in memory go to the
+// node-space band LU / compliance-form band Cholesky of run_gradient3, which needs less memory per image.  A shape the
+// band solvers refuse as well (above 430² for the band LU, 136² for the band Cholesky) goes back to the fronts with their
+// large-front variants; a failure there is final, and an image whose workspace does not fit returns BPLTV_ERR_ALLOC with
+// the size it needs.
+// The patch sumregs_gradient_reg (:195-262, row-scaled, not symmetric) takes the band LU first, as it always has; a shape
+// the band LU refuses goes to the LU form of the fronts (shared-memory fronts, then the large-front variants).  Solver 1
+// keeps it on the band LU; BPLTV_SUMREGS_PATCH_REG_ND=1 sends it to the fronts' LU at every size they take.
 template <typename Real>
 static int run_sumregs_gradient(Dev &d, const Grad3Problem<Real> &gp, int solver, int maxit, cudaStream_t st,
                                 double *d_grad_out)
 {
     if (solver == 0) solver = env_int("BPLTV_GRAD_SOLVER", 0);
     d.last_grad = Dev::GRAD_NONE;
-    const bool fronts = solver != 1 && gp.M == gp.N && !(gp.regularised && gp.alpha_maps);
+    const bool patch_reg = gp.regularised && gp.alpha_maps;
+    const bool fronts = solver != 1 && gp.M == gp.N && !patch_reg;
     auto nd = [&](bool large) {
         if (!d.nd3) d.nd3 = nd_work_create();
         int rc;
@@ -1186,6 +1190,7 @@ static int run_sumregs_gradient(Dev &d, const Grad3Problem<Real> &gp, int solver
             np.u = gp.u; np.ubar = gp.ubar; np.prec = (int)sizeof(Real) * 8; np.M = gp.M; np.N = gp.N; np.O = gp.O;
             for (int k = 0; k < 3; ++k) np.alpha[k] = gp.alpha[k];
             np.gamma = gp.gamma; np.tol = 0.0; np.maxit = maxit; np.large_fronts = large;
+            np.alpha_maps = gp.alpha_maps; np.lm = gp.lm; np.ln = gp.ln;
             rc = nd_run_gradient3_reg(d.nd3, np, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
         } else {
             Nd3mProblem np;
@@ -1198,14 +1203,29 @@ static int run_sumregs_gradient(Dev &d, const Grad3Problem<Real> &gp, int solver
         if (rc == 0) d.last_grad = Dev::GRAD_SR_ND;
         return rc;
     };
+    auto band = [&]() {
+        const int rc = run_gradient3<Real>(d.grad3, gp, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
+        if (rc == 0) d.last_grad = Dev::GRAD_SR_BAND;
+        return rc;
+    };
+    if (patch_reg && solver != 1 && gp.M == gp.N) {
+        const bool nd_first = env_int("BPLTV_SUMREGS_PATCH_REG_ND", 0) != 0;
+        int rc = nd_first ? -1 : band();
+        if (rc == -1) {
+            rc = nd(false);
+            if (rc == -1) rc = nd(true);
+            if (rc != 0 && rc != -1) d.grad3.err = nd_work_error(d.nd3);
+        }
+        if (rc == -1 && nd_first) rc = band();      // images the fronts do not take (below 8²)
+        return rc;
+    }
     int nd_rc = -1;
     if (fronts) {
         nd_rc = nd(false);
         if (nd_rc == 0) return 0;
         if (nd_rc != -1 && nd_rc != BPLTV_ERR_ALLOC) { d.grad3.err = nd_work_error(d.nd3); return nd_rc; }
     }
-    int rc = run_gradient3<Real>(d.grad3, gp, d.sm_count, d.smem_optin, st, d_grad_out, &d.launches);
-    if (rc == 0) d.last_grad = Dev::GRAD_SR_BAND;
+    int rc = band();
     if (rc == -1 && fronts) {
         if (nd_rc == -1) rc = nd(true);
         else rc = nd_rc;        // the fronts took the shape but their workspace did not fit: say so, with its size

@@ -76,7 +76,7 @@ struct NdBuf {
 struct NdWork {
     std::string err;
     NdPlan plan;
-    NdBuf pix, off, off3, lvl, vec, posg, foff, totals, ast, L, U0, U1, UV0, UV1, scr, info, out_img, relres, relres_max;
+    NdBuf pix, off, off3, lvl, vec, posg, foff, totals, ast, L, U0, U1, UV0, UV1, scr, info, rstate, out_img, relres, relres_max;
     std::vector<long long> h_totals;
     size_t budget_cached = 0;
     // what the last call saw (statistics)
@@ -89,7 +89,8 @@ struct NdWork {
     {
         slots_key_n = slots_key_node = slots_key_want = -1;
         plan.release();
-        NdBuf *all[] = {&pix, &off, &off3, &lvl, &vec, &posg, &foff, &totals, &ast, &L, &U0, &U1, &UV0, &UV1, &scr, &info, &out_img, &relres, &relres_max};
+        NdBuf *all[] = {&pix, &off, &off3, &lvl, &vec, &posg, &foff, &totals, &ast, &L, &U0, &U1, &UV0, &UV1, &scr, &info, &rstate,
+                        &out_img, &relres, &relres_max};
         for (NdBuf *b : all) b->release();
     }
 };
@@ -209,6 +210,40 @@ static int nd_kernel_attributes(NdWork &w, size_t fsmem, size_t ssmem, size_t fs
     return 0;
 }
 
+using NdFactorKernel = void (*)(NdDev, int, int, double, int);
+
+// Opt-in shared memory of the LU factorisation kernels (nd_lu_factor_*): fsmem for the shared-memory panels, fsmem_large
+// for the panels in global memory (0: none of the level's)
+static int nd_lu_kernel_attributes(NdWork &w, size_t fsmem, size_t fsmem_large)
+{
+    static std::mutex mu;
+    static int have[64][2] = {};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    dev = std::max(0, std::min(63, dev));
+    std::lock_guard<std::mutex> lock(mu);
+    cudaError_t e = cudaSuccess;
+    const size_t want[2] = {fsmem, fsmem_large};
+    const NdFactorKernel ks[2][4] = {{nd_lu_factor_kernel, nd_lu_factor8_kernel, nd_lu_factor_cluster_kernel, nd_lu_factor8_cluster_kernel},
+                                        {nd_lu_factor_large_kernel, nd_lu_factor8_large_kernel, nd_lu_factor_large_cluster_kernel,
+                                         nd_lu_factor8_large_cluster_kernel}};
+    for (int g = 0; g < 2 && e == cudaSuccess; ++g) {
+        if (want[g] == 0 || have[dev][g] >= (int)want[g]) continue;
+        for (int k = 0; k < 4 && e == cudaSuccess; ++k) {
+            e = cudaFuncSetAttribute(ks[g][k], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)want[g]);
+            if (e == cudaSuccess && k >= 2) e = cudaFuncSetAttribute(ks[g][k], cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+        }
+        if (e == cudaSuccess) have[dev][g] = (int)want[g];
+    }
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        char buf[128];
+        snprintf(buf, sizeof buf, " (dynamic shared memory of the LU factorisation: %zu / %zu B)", fsmem, fsmem_large);
+        return nd_fail(w, -2, std::string("nested-dissection kernel attributes: ") + cudaGetErrorString(e) + buf);
+    }
+    return 0;
+}
+
 // Dynamic shared memory a front kernel may ask for: the opt-in maximum per block less the static shared memory of the
 // factorisation kernels (their block-step flags, 16 B), which the opt-in maximum also has to hold.
 static size_t nd_dynamic_optin(size_t smem_optin)
@@ -237,9 +272,9 @@ static size_t nd_large_limit(size_t smem_optin)
 // Launch plan of every level of the tree for `mb` unknowns per pixel at most (`fsz` typical): CTA sizes, shared memory of
 // the largest front (worst case: mb unknowns on every pixel), kernel attributes.  -1: a front does not fit in shared
 // memory and `large` is not set (the caller lets a band solver try first); with `large`, such levels take the
-// large-front variants.
+// large-front variants.  lu: the LU form (nd_level_lu: every level's factorisation on the generic LU kernels).
 static int nd_prepare_levels(NdWork &w, const NdSymbolic &sym, int mb, double fsz, int O, size_t smem_optin, bool large,
-                             std::vector<NdLevelPlan> &plan, std::vector<char> &plan_small)
+                             std::vector<NdLevelPlan> &plan, std::vector<char> &plan_small, bool lu = false)
 {
     const int nsteps = sym.nsteps();
     // CTA size of the generic front factorisation: a stack of many images has fronts for every SM several times over, and
@@ -260,18 +295,29 @@ static int nd_prepare_levels(NdWork &w, const NdSymbolic &sym, int mb, double fs
         plan_small[s] = plan[s].small;
         if (plan[s].small) { fsmem_small = std::max(fsmem_small, plan[s].smem_f); ssmem_small = std::max(ssmem_small, plan[s].smem_s); }
         // every level can also run on the generic kernels
+        if (lu) nd_level_lu(plan[s], smem_optin);
         if (!nd_level_large(plan[s], limit, smem_optin, large)) return -1;
         size_t &f = plan[s].large_f ? fsmem_large : fsmem, &g = plan[s].large_s ? ssmem_large : ssmem;
         f = std::max(f, nd_level_smem_f(plan[s]));
         g = std::max(g, nd_level_smem_s(plan[s]));
     }
+    if (lu) {
+        const int rc = nd_kernel_attributes(w, 0, ssmem, 0, ssmem_small, smem_optin, 0, 0, ssmem_large);
+        return rc != 0 ? rc : nd_lu_kernel_attributes(w, fsmem, fsmem_large);
+    }
     return nd_kernel_attributes(w, fsmem, ssmem, fsmem_small, ssmem_small, smem_optin, 0, fsmem_large, ssmem_large);
 }
 
-using NdFactorKernel = void (*)(NdDev, int, int, double, int);
 // the generic factorisation kernel of a level: block width, where the panel lives, alone or shared by a cluster
 static NdFactorKernel nd_factor_kernel_of(const NdLevelPlan &lp, bool cluster)
 {
+    if (lp.lu) {
+        if (lp.large_f)
+            return lp.nb != ND_NB ? (cluster ? nd_lu_factor8_large_cluster_kernel : nd_lu_factor8_large_kernel)
+                                  : (cluster ? nd_lu_factor_large_cluster_kernel : nd_lu_factor_large_kernel);
+        return lp.nb != ND_NB ? (cluster ? nd_lu_factor8_cluster_kernel : nd_lu_factor8_kernel)
+                              : (cluster ? nd_lu_factor_cluster_kernel : nd_lu_factor_kernel);
+    }
     if (lp.large_f)
         return lp.nb != ND_NB ? (cluster ? nd_factor8_large_cluster_kernel : nd_factor8_large_kernel)
                               : (cluster ? nd_factor_large_cluster_kernel : nd_factor_large_kernel);
@@ -377,7 +423,8 @@ static int nd_factor_cta_threads(const NdLevelPlan &lp, int cnt, int sm_count)
     return std::min(lp.threads_f, 32 * cap);
 }
 
-// one launch per level: assemble + partial Cholesky of every front of the wave's `cnt` images
+// one launch per level: assemble + partial Cholesky (LU form: partial LU, on the generic kernels at every level) of
+// every front of the wave's `cnt` images
 static void nd_launch_factor(const NdDev &nd, std::vector<NdLevelPlan> &plan, const std::vector<char> &plan_small,
                              const NdSymbolic &sym, int mb, int cnt, int sm_count, double guard, cudaStream_t st, long long *launches)
 {
@@ -387,7 +434,7 @@ static void nd_launch_factor(const NdDev &nd, std::vector<NdLevelPlan> &plan, co
     for (int s = 0; s < nsteps; ++s) plan[s].small = plan_small[s] && (long long)plan[s].nfr * cnt >= 4LL * sm_count;
     for (int s = 0; s < nsteps; ++s) {
         const NdLevelPlan &lp = plan[s];
-        if (lp.small)
+        if (lp.small && !lp.lu)
             nd_factor_small_kernel<<<dim3((lp.nfr + ND_SMALL_WARPS - 1) / ND_SMALL_WARPS, cnt), 32 * ND_SMALL_WARPS, lp.smem_f, st>>>(
                 nd, lp.t0, lp.nfr, s & 1, guard, lp.arena_f);
         else {
@@ -401,11 +448,13 @@ static void nd_launch_factor(const NdDev &nd, std::vector<NdLevelPlan> &plan, co
     *launches += nsteps;
 }
 
-// L y = b up the tree, Lᵀ x = y down: `vec` (per image, `stride` doubles apart) is overwritten by the solution
-static void nd_launch_solve(const NdDev &nd, const std::vector<NdLevelPlan> &plan, int cnt, double *vec, size_t stride,
-                            cudaStream_t st, long long *launches)
+// L y = b up the tree, Lᵀ x = y down: `vec` (per image, `stride` doubles apart) is overwritten by the solution.
+// lu (LU form, nd_lu_factor_body): the backward sweep solves U x = y on the transposed rows of U instead.
+static void nd_launch_solve(const NdDev &nd_fwd, const std::vector<NdLevelPlan> &plan, int cnt, double *vec, size_t stride,
+                            cudaStream_t st, long long *launches, bool lu = false)
 {
     const int nsteps = (int)plan.size();
+    NdDev nd = nd_fwd;
     for (int s = 0; s < nsteps; ++s) {
         const NdLevelPlan &lp = plan[s];
         if (lp.small)
@@ -416,6 +465,7 @@ static void nd_launch_solve(const NdDev &nd, const std::vector<NdLevelPlan> &pla
         else
             nd_fwd_kernel<<<dim3(lp.nfr, cnt), lp.threads_s, nd_solve_smem(lp.nFw), st>>>(nd, lp.t0, s & 1, vec, stride);
     }
+    if (lu) nd.L += nd.L_stride / 2;
     for (int s = nsteps - 1; s >= 0; --s) {
         const NdLevelPlan &lp = plan[s];
         if (lp.small)
@@ -607,17 +657,22 @@ static int run_gradient_nd(NdWork &w, const NdProblem &gp, int sm_count, size_t 
 }
 
 // ---------------------------------------------------------------------------
-// scalar sumregs_gradient_reg on the same solver (nd_sumregs.cuh): node space, one unknown per node, W = 2
+// sumregs_gradient_reg on the same solver (nd_sumregs.cuh): node space, one unknown per node, W = 2.  Scalar parameter:
+// the Cholesky of the fronts.  Patch parameter (alpha_maps, row-scaled): the LU of the fronts (nd_lu_factor_body), with
+// the band LU's refinement (at most 3 steps, stopped when a step no longer gains a factor 4) and backward-error test.
 // ---------------------------------------------------------------------------
 template <typename Real>
 static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, size_t smem_optin, cudaStream_t st,
                                 double *d_grad_out, long long *launches)
 {
     const Real *gp_u = static_cast<const Real *>(gp.u), *gp_ubar = static_cast<const Real *>(gp.ubar);
-    const int n = gp.M, N = gp.M * gp.N, nops = 3, ng = 1;
+    const Real *amaps = static_cast<const Real *>(gp.alpha_maps);
+    const bool lu = amaps != nullptr;
+    const int n = gp.M, N = gp.M * gp.N, nops = 3, ng = lu ? gp.lm * gp.ln : 1;
     smem_optin = nd_dynamic_optin(smem_optin);
     if (gp.M != gp.N) return nd_fail(w, -1, "square images required");
     if (n < 8) return -1;                                   // tiny images: the band LU
+    if (nops * ng > 1024) return nd_fail(w, -1, "lambda grid larger than 1024 entries is not supported");
     {
         const int rc = nd_build_plan(w.plan, n, ND3_W, st, w.err);
         if (rc != 0) return rc;
@@ -628,17 +683,18 @@ static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, s
     std::vector<NdLevelPlan> plan;
     std::vector<char> plan_small;
     {
-        const int rc = nd_prepare_levels(w, sym, 1, 1.0, gp.O, smem_optin, gp.large_fronts, plan, plan_small);
+        const int rc = nd_prepare_levels(w, sym, 1, 1.0, gp.O, smem_optin, gp.large_fronts, plan, plan_small, lu);
         if (rc != 0) return rc;
     }
     const long long *t1 = w.plan.tot1;
-    const size_t pix_stride = (size_t)LU_PLANES * N, ast_stride = (size_t)ND3_NH * N;
+    const size_t pix_stride = (size_t)LU_PLANES * N, ast_stride = (size_t)(lu ? ND3_NH2 : ND3_NH) * N;
     const size_t Ls = ((size_t)t1[0] + 1) & ~(size_t)1, Us = ((size_t)t1[1] + 1) & ~(size_t)1, UVs = ((size_t)t1[2] + 1) & ~(size_t)1;
     const size_t scr_stride = nd_scratch_doubles(plan, sm_count);
-    const size_t per_slot = (pix_stride + ast_stride + Ls + 2 * Us + 2 * UVs + scr_stride) * 8 + 16;
+    const size_t per_slot = (pix_stride + ast_stride + (lu ? 2 : 1) * Ls + 2 * Us + 2 * UVs + scr_stride + (lu ? 2 : 0)) * 8 + 16;
     w.last_bytes_per_image = per_slot;
     int slots = std::min(gp.O, 256);
-    if (w.slots_key_n == n && w.slots_key_node == 3 && w.slots_key_want == slots) {
+    const int key = lu ? 4 : 3;
+    if (w.slots_key_n == n && w.slots_key_node == key && w.slots_key_want == slots) {
         slots = w.slots_cached;
     } else {
         const int want = slots;
@@ -647,7 +703,7 @@ static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, s
         const size_t have = w.pix.bytes + w.ast.bytes + w.L.bytes + w.U0.bytes + w.U1.bytes;
         const size_t budget = (free_b + have) / 2;
         slots = (int)std::min<size_t>((size_t)slots, std::max<size_t>(1, budget / per_slot));
-        w.slots_key_n = n; w.slots_key_node = 3; w.slots_key_want = want; w.slots_cached = slots;
+        w.slots_key_n = n; w.slots_key_node = key; w.slots_key_want = want; w.slots_cached = slots;
     }
     auto need = [&](NdBuf &b, size_t bytes, const char *what) -> int {
         const cudaError_t e = b.ensure(bytes);
@@ -660,7 +716,8 @@ static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, s
     if ((rc = need(w.out_img, (size_t)gp.O * nops * ng * 8, "per-image gradients"))) return rc;
     if ((rc = need(w.relres, (size_t)gp.O * 8, "residuals"))) return rc;
     if ((rc = need(w.relres_max, 16, "residual maximum"))) return rc;
-    if ((rc = need(w.L, Ls * 8 * slots, "factors"))) return rc;
+    if ((rc = need(w.L, (lu ? 2 : 1) * Ls * 8 * slots, "factors"))) return rc;
+    if (lu && (rc = need(w.rstate, (size_t)16 * slots, "refinement state"))) return rc;
     if ((rc = need(w.U0, Us * 8 * slots, "update matrices"))) return rc;
     if ((rc = need(w.U1, Us * 8 * slots, "update matrices"))) return rc;
     if ((rc = need(w.UV0, UVs * 8 * slots, "update vectors"))) return rc;
@@ -672,7 +729,7 @@ static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, s
     ws.n = n; ws.N = N; ws.bw = 0; ws.bwx = 0; ws.LD = 0; ws.use_pin = 0; ws.nops = nops;
     Lu3Params pr;
     for (int k = 0; k < 3; ++k) pr.alpha[k] = gp.alpha[k];
-    pr.gamma = gp.gamma; pr.lm = 1; pr.ln = 1; pr.refine = 0;
+    pr.gamma = gp.gamma; pr.lm = lu ? gp.lm : 1; pr.ln = lu ? gp.ln : 1; pr.refine = lu ? 3 : 0;
 
     NdDev nd;
     nd.n = n; nd.N = N; nd.W = ND3_W; nd.nnb = sym.nnb; nd.nh = nd_nh(ND3_W); nd.mb = 1;
@@ -683,37 +740,41 @@ static int run_gradient3_nd_reg(NdWork &w, const Nd3Problem &gp, int sm_count, s
     nd.posg = (int *)w.plan.d_posg1; nd.posg_stride = 0;
     nd.foff = (long long *)w.plan.d_foff1; nd.foff_stride = 0;
     nd.totals = nullptr;
-    nd.L = (double *)w.L.p; nd.L_stride = Ls;
+    nd.L = (double *)w.L.p; nd.L_stride = (lu ? 2 : 1) * Ls;      // LU form: L, then Uᵀ
     nd.U[0] = (double *)w.U0.p; nd.U[1] = (double *)w.U1.p; nd.U_stride = Us;
     nd.UV[0] = (double *)w.UV0.p; nd.UV[1] = (double *)w.UV1.p; nd.UV_stride = UVs;
     nd.ast = (const double *)w.ast.p; nd.ast_stride = ast_stride;
     nd.info = (int *)w.info.p;
     nd.scr = (double *)w.scr.p; nd.scr_stride = scr_stride;
+    double *rstate = lu ? (double *)w.rstate.p : nullptr;
 
-    const double tol = gp.tol > 0 ? gp.tol : 1e300;
-    const int refine = gp.maxit > 0 ? std::min(gp.maxit, 8) : 1;
+    // the patch form: the band LU's backward-error tolerance and refinement (lu3_solve_kernel)
+    const double tol = lu ? 1e-11 : (gp.tol > 0 ? gp.tol : 1e300);
+    const int refine = lu ? pr.refine : (gp.maxit > 0 ? std::min(gp.maxit, 8) : 1);
     const int chunks = std::max(1, std::min(64, (N + 255) / 256));
     for (int img0 = 0; img0 < gp.O; img0 += slots) {
         const int cnt = std::min(slots, gp.O - img0);
         cudaMemsetAsync(w.ast.p, 0, ast_stride * 8 * cnt, st);
         cudaMemsetAsync(w.info.p, 0, (size_t)16 * cnt, st);
         lu3_classify_kernel<Real><<<dim3(cnt, chunks), 256, 0, st>>>(ws, pr.gamma, gp_u, gp_ubar, img0);
-        nd3_stencil_kernel<<<dim3(cnt, chunks), 256, 0, st>>>(ws, pr, (double *)w.ast.p, ast_stride);
+        if (lu) nd3_stencil_map_kernel<Real><<<dim3(cnt, chunks), 256, 0, st>>>(ws, pr, amaps, (double *)w.ast.p, ast_stride);
+        else nd3_stencil_kernel<<<dim3(cnt, chunks), 256, 0, st>>>(ws, pr, (double *)w.ast.p, ast_stride);
         *launches += 2;
         nd_launch_factor(nd, plan, plan_small, sym, 1, cnt, sm_count, 0.0, st, launches);
         double *p = ws.pix + (size_t)LU_PL_P * N, *work = ws.pix + (size_t)LU_PL_WORK * N;
-        nd_launch_solve(nd, plan, cnt, p, pix_stride, st, launches);
-        nd3_residual_kernel<Real><<<cnt, 1024, 0, st>>>(ws, pr, (double *)w.relres.p, img0);
+        nd_launch_solve(nd, plan, cnt, p, pix_stride, st, launches, lu);
+        nd3_residual_kernel<Real><<<cnt, 1024, 0, st>>>(ws, pr, (double *)w.relres.p, img0, amaps, rstate, 0);
         for (int it = 0; it < refine; ++it) {
-            nd_launch_solve(nd, plan, cnt, work, pix_stride, st, launches);
-            nd3_axpy_kernel<<<dim3(cnt, chunks), 256, 0, st>>>(ws);
-            nd3_residual_kernel<Real><<<cnt, 1024, 0, st>>>(ws, pr, (double *)w.relres.p, img0);
+            nd_launch_solve(nd, plan, cnt, work, pix_stride, st, launches, lu);
+            nd3_axpy_kernel<<<dim3(cnt, chunks), 256, 0, st>>>(ws, rstate);
+            nd3_residual_kernel<Real><<<cnt, 1024, 0, st>>>(ws, pr, (double *)w.relres.p, img0, amaps, rstate, it + 1);
         }
-        nd3_finish_kernel<<<cnt, 1024, 0, st>>>(ws, pr, (const int *)w.info.p, tol, (double *)w.out_img.p, (double *)w.relres.p, img0);
+        nd3_finish_kernel<Real><<<cnt, 1024, 0, st>>>(ws, pr, (const int *)w.info.p, tol, (double *)w.out_img.p, (double *)w.relres.p,
+                                                      img0, amaps);
         *launches += 2 + 2 * refine;
     }
-    nd_reduce_kernel<<<1, 32, 0, st>>>((double *)w.out_img.p, (double *)w.relres.p, gp.O, nops * ng, d_grad_out,
-                                       (double *)w.relres_max.p);
+    nd_reduce_kernel<<<(nops * ng + 31) / 32, 32, 0, st>>>((double *)w.out_img.p, (double *)w.relres.p, gp.O, nops * ng, d_grad_out,
+                                                         (double *)w.relres_max.p);
     *launches += 1;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return nd_fail(w, -2, std::string("nested-dissection kernel launch failed: ") + cudaGetErrorString(e));

@@ -24,8 +24,10 @@ struct NdProblem {
     bool large_fronts;          // fronts beyond shared memory take the large-front variants instead of returning -1
 };
 
-// scalar sumregs_gradient_reg of /root/reference/src/SumRegsLearningFunction.jl:112-167 (three difference operators,
-// symmetric node-space system, coupling radius 2) for a stack of O images on the device
+// sumregs_gradient_reg of /root/reference/src/SumRegsLearningFunction.jl for a stack of O images on the device (three
+// difference operators, node space, coupling radius 2): scalar (:112-167, symmetric: Cholesky of the fronts) or patch
+// (:195-262, alpha_maps: rows scaled by a different map per operator, LU of the fronts, refined and checked as the band
+// LU does — tol and maxit are not used then)
 struct Nd3Problem {
     const void *u, *ubar;
     int prec;
@@ -35,6 +37,8 @@ struct Nd3Problem {
     double tol;                 // backward error above which the result is poisoned with NaN (≤ 0: never)
     int maxit;                  // refinement steps (≤ 0: default)
     bool large_fronts;          // fronts beyond shared memory take the large-front variants instead of returning -1
+    const void *alpha_maps = nullptr;     // 3 maps of M·N (patch) or nullptr (scalar: alpha[3])
+    int lm = 1, ln = 1;                   // the patch grid
 };
 
 // sumregs_gradient (non-regularised; scalar :264-327, patch :330-407) in multiplier space: 3-6 unknowns per pixel,
@@ -60,7 +64,8 @@ const double *nd_work_relres_max(const NdWork *w);      // device pointer: worst
 // negatives: bpltv_status (BPLTV_ERR_ALLOC: the workspace of one image does not fit; the message names its size)
 int nd_run_gradient(NdWork *w, const NdProblem &gp, int sm_count, size_t smem_optin, cudaStream_t st, double *d_grad_out,
                     long long *launches);
-// d_grad_out: 3 doubles (one per operator).  Use a workspace of its own (the plan is keyed by the coupling radius).
+// d_grad_out: 3·lm·ln doubles, [operator][patch] (3 for the scalar parameter).  Use a workspace of its own (the plan is
+// keyed by the coupling radius).
 int nd_run_gradient3_reg(NdWork *w, const Nd3Problem &gp, int sm_count, size_t smem_optin, cudaStream_t st, double *d_grad_out,
                          long long *launches);
 

@@ -15,6 +15,8 @@
 //                        U stays in the level's pool for the parent; L11 and L21 are kept
 //   nd_fwd_kernel      L y = b   up the tree (children's update vectors are summed in a fixed order)
 //   nd_bwd_kernel      Lᵀ x = y  down the tree
+//   nd_lu_factor_*     the same for an unsymmetric matrix of the same sparsity: partial LU without pivoting, L and
+//                      Uᵀ in the column layout of L, so that nd_fwd / nd_bwd solve with them unchanged
 //
 // Every sum has a fixed order: results are deterministic, independent of the grid shape of the launch.
 // Fronts live in global memory (the working set of a level is L2-resident); a front of the top levels of a
@@ -266,10 +268,11 @@ static __device__ __forceinline__ double *nd_col(double *L, double *U, int nP, i
 
 static __host__ __device__ __forceinline__ int nd_panel_pitch(int nFmax) { return (nFmax + 31) & ~31; }
 // dynamic shared memory of nd_factor_kernel (bytes): S0, S, reciprocal diagonal, column floors, panel P (NB × pitch;
-// not on the large-front variants, which keep it in global memory), the child map (ints)
-static inline size_t nd_factor_smem(int nFmax, int nRchild_max, int nb = ND_NB, bool panel_global = false)
+// not on the large-front variants, which keep it in global memory), the child map (ints).  lu: nd_lu_factor_body, whose
+// two panels (L21 and U12ᵀ) take twice the room.
+static inline size_t nd_factor_smem(int nFmax, int nRchild_max, int nb = ND_NB, bool panel_global = false, bool lu = false)
 {
-    return (size_t)(2 * nb * nb + 2 * nb + (panel_global ? 0 : nb * nd_panel_pitch(nFmax))) * sizeof(double) +
+    return (size_t)(2 * nb * nb + 2 * nb + (panel_global ? 0 : (lu ? 2 : 1) * nb * nd_panel_pitch(nFmax))) * sizeof(double) +
            (((size_t)nRchild_max * sizeof(int) + 15) & ~(size_t)15);
 }
 
@@ -529,6 +532,296 @@ __global__ void __launch_bounds__(512) nd_factor_large_kernel(NdDev nd, int t0, 
 __global__ void __launch_bounds__(512) nd_factor_large_cluster_kernel(NdDev nd, int t0, int par, double guard, int nFmax) { nd_factor_body<true, ND_NB, true>(nd, t0, par, guard, nFmax); }
 __global__ void __launch_bounds__(512) nd_factor8_large_kernel(NdDev nd, int t0, int par, double guard, int nFmax) { nd_factor_body<false, 8, true>(nd, t0, par, guard, nFmax); }
 __global__ void __launch_bounds__(512) nd_factor8_large_cluster_kernel(NdDev nd, int t0, int par, double guard, int nFmax) { nd_factor_body<true, 8, true>(nd, t0, par, guard, nFmax); }
+
+// ===========================================================================
+// LU form: the same fronts for an UNSYMMETRIC matrix with the sparsity of the symmetric one (the row-scaled patch
+// sum-of-regularisers system, nd_sumregs.cuh).  No pivoting: every term of that matrix is a positive diagonal times a
+// PSD matrix; with equal maps it is D·SPD, and a symmetric reordering P(D·S)Pᵀ keeps that form, so its leading minors
+// stay positive.  A zero or non-finite pivot sets the breakdown flag; the caller's backward-error test does the rest.
+//
+// Storage: F = L U with L unit lower.  L (nd.L) holds L's first nP columns, its unit diagonal written out; Ut holds U's
+// first nP ROWS, transposed, in the same nF × nP column layout (column c = row c of U, entries r ≥ c, diagonal
+// included); the update matrix is the whole nR × nR Schur complement.  A slot's factor pool is twice the Cholesky's:
+// L in its first half, Ut at the same offsets in its second (nd.L_stride / 2 further).  The forward sweep of nd_fwd_body
+// on L solves L y = b (its pivots are exactly 1), the backward sweep of nd_bwd_body on Ut solves U x = y: the solve
+// kernels are the Cholesky's, launched with nd.L moved to the second half for the backward sweep.
+// The ast of this form has 2·nh − 1 blocks per pixel: [0] A[p, p] (the whole block), [h] A[p + d_h, p] as in the
+// symmetric form, [nh − 1 + h] A[p, p + d_h].
+// ===========================================================================
+constexpr double ND_DMAX = 1.7976931348623157e308;
+
+// entry (R, C) of the front while it is factorised: pivot columns on or below the diagonal in L, pivot rows right of
+// the diagonal in Ut, the rest in the update matrix
+static __device__ __forceinline__ double *nd_lu_at(double *L, double *Ut, double *U, int nP, int nF, int nR, int R, int C)
+{
+    if (C < nP && R >= C) return L + (size_t)C * nF + R;
+    if (R < nP) return Ut + (size_t)R * nF + C;
+    return U + (size_t)(C - nP) * nR + (R - nP);
+}
+
+// One warp: S0 (NB×NB row-major, identity padded beyond nb) → its LU without pivoting in S (row-major: the multipliers
+// of L below the diagonal, U on and above it) and the reciprocals of U's diagonal in dinv.  Rows across lanes, columns
+// through shuffles.  A zero or non-finite pivot sets `bad` and is replaced by 1, so that the step completes.
+template <int NB>
+static __device__ void nd_lu_diag_block(const double *S0, double *S, double *dinv, int nb, int lane, int &bad)
+{
+    double row[NB];
+    const int lr = lane < NB ? lane : NB - 1;
+#pragma unroll
+    for (int c = 0; c < NB; ++c) row[c] = S0[lr * NB + c];
+    double dinv_own = 1.0;
+#pragma unroll
+    for (int c = 0; c < NB; ++c) {
+        double d = __shfl_sync(0xffffffffu, row[c], c);
+        if (!(fabs(d) > 0.0 && fabs(d) <= ND_DMAX)) {
+            if (lane == 0 && c < nb) bad = 1;
+            d = 1.0;
+        }
+        const double inv = 1.0 / d;
+        const double l = row[c] * inv;
+#pragma unroll
+        for (int c2 = c + 1; c2 < NB; ++c2) {
+            const double uc2 = __shfl_sync(0xffffffffu, row[c2], c);
+            if (lane > c) row[c2] = fma(-l, uc2, row[c2]);
+        }
+        if (lane == c) { row[c] = d; dinv_own = inv; }
+        else if (lane > c) row[c] = l;
+    }
+    if (lane < NB) {
+#pragma unroll
+        for (int c = 0; c < NB; ++c) S[lane * NB + c] = row[c];
+        dinv[lane] = dinv_own;
+    }
+    __syncwarp();
+}
+
+// assemble + partial LU of the fronts of one level; CL, NB and PG as nd_factor_body (a cluster's CTAs form the diagonal
+// block and both panels redundantly and share the tiles of the trailing update: the same bits for every cluster size;
+// the panels in global memory give the bits of the shared-memory kernel at the same NB).  Blocked right-looking, per step:
+// the diagonal block by one warp (nd_lu_diag_block), L21 = F21 U11⁻¹ and U12ᵀ = (L11⁻¹ F12)ᵀ by substitution with one
+// thread per row of both panels, F22 −= L21 U12 over ALL 32×32 tiles of the trailing matrix.
+template <bool CL, int NB, bool PG = false>
+static __device__ __forceinline__ void nd_lu_factor_body(const NdDev &nd, int t0, int par, int nFmax)
+{
+    ND_DYN_SMEM(sm);
+    const int PR = nd_panel_pitch(nFmax);
+    double *S0 = sm, *S = sm + NB * NB, *dinv = sm + 2 * NB * NB;
+    double *PL = PG ? nd.scr + nd.scr_stride * blockIdx.y + (size_t)blockIdx.x * 2 * NB * PR : dinv + 2 * NB;
+    double *PU = PL + (size_t)NB * PR;
+    int *umap = reinterpret_cast<int *>(PG ? dinv + 2 * NB : PU + (size_t)NB * PR);
+    const int tid = threadIdx.x, T = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarps = T >> 5;
+    int crank = 0, csize = 1;
+    if (CL) {
+        cooperative_groups::cluster_group cluster = cooperative_groups::this_cluster();
+        crank = (int)cluster.block_rank(); csize = (int)cluster.num_blocks();
+    }
+    auto csync = [&]() { if (CL) cooperative_groups::this_cluster().sync(); else __syncthreads(); };
+    const int gtid = crank * T + tid, GT = csize * T;
+    const int t = t0 + blockIdx.x / csize, slot = blockIdx.y;
+    const NdFront f = nd.fronts[t];
+    const int *pos = nd.posg + nd.posg_stride * slot + f.pix0 + t;
+    const long long *foff = nd.foff + nd.foff_stride * slot;
+    const int nP = pos[f.npiv], nF = pos[f.npiv + f.nring], nR = nF - nP;
+    double *L = nd.L + nd.L_stride * slot + foff[4 * (size_t)t];
+    double *Ut = L + nd.L_stride / 2;
+    double *U = nd.U[par] + nd.U_stride * slot + foff[4 * (size_t)t + 1];
+    const double *ast = nd.ast + nd.ast_stride * slot;
+    const int MB = nd.mb, MB2 = MB * MB, NH2 = 2 * nd.nh - 1;
+
+    // ---- zero
+    for (size_t k = gtid; k < (size_t)nF * nP; k += GT) { L[k] = 0.0; Ut[k] = 0.0; }
+    for (size_t k = gtid; k < (size_t)nR * nR; k += GT) U[k] = 0.0;
+    csync();
+    // ---- original entries of the pivot rows and columns (each pixel pair once: by the earlier pixel of the front)
+    {
+        const int ne = nd.nnb + 1;
+        for (int idx = gtid; idx < f.npiv * ne; idx += GT) {
+            const int kp = idx / ne, e = idx - kp * ne;
+            const int p = nd.pixlist[f.pix0 + kp];
+            const int a0 = pos[kp], mp = pos[kp + 1] - a0;
+            if (e == 0) {
+                const double *blk = ast + (size_t)p * NH2 * MB2;       // blk[be·MB + al] = F(a0 + be, a0 + al)
+                for (int al = 0; al < mp; ++al)
+                    for (int be = 0; be < mp; ++be) {
+                        if (be >= al) L[(size_t)(a0 + al) * nF + a0 + be] = blk[be * MB + al];
+                        else Ut[(size_t)(a0 + be) * nF + a0 + al] = blk[be * MB + al];
+                    }
+            } else {
+                const int kq = nd.nbr[f.nbr0 + kp * nd.nnb + (e - 1)];
+                if (kq <= kp) continue;
+                const int q = nd.pixlist[f.pix0 + kq];
+                const int b0 = pos[kq], mq = pos[kq + 1] - b0;
+                const int h = 1 + ((e - 1) >> 1);
+                const bool fwd = ((e - 1) & 1) == 0;       // q = p + d_h, else p = q + d_h
+                const double *lo = ast + ((size_t)(fwd ? p : q) * NH2 + h) * MB2;              // A[· + d_h, ·]
+                const double *up = ast + ((size_t)(fwd ? p : q) * NH2 + nd.nh - 1 + h) * MB2;  // A[·, · + d_h]
+                const double *bqp = fwd ? lo : up, *bpq = fwd ? up : lo;   // A[q, p], A[p, q]: [row unknown · MB + column unknown]
+                for (int al = 0; al < mp; ++al)
+                    for (int be = 0; be < mq; ++be) {
+                        L[(size_t)(a0 + al) * nF + b0 + be] = bqp[be * MB + al];
+                        Ut[(size_t)(a0 + al) * nF + b0 + be] = bpq[al * MB + be];
+                    }
+            }
+        }
+    }
+    csync();
+    // ---- extend-add: the children's whole update matrices, one child after the other (fixed order)
+    for (int ci = 0; ci < 2; ++ci) {
+        const int c = ci == 0 ? f.child0 : f.child1;
+        if (c < 0) continue;
+        const NdFront cf = nd.fronts[c];
+        const int *cpos = nd.posg + nd.posg_stride * slot + cf.pix0 + c + cf.npiv;
+        const int cnP = cpos[0], cnR = cpos[cf.nring] - cnP;
+        for (int k = tid; k < cf.nring; k += T) {
+            const int r0 = cpos[k] - cnP, m = cpos[k + 1] - cpos[k];
+            const int R0 = pos[nd.cmap[cf.cmap0 + k]];
+            for (int al = 0; al < m; ++al) umap[r0 + al] = R0 + al;
+        }
+        __syncthreads();
+        const double *cU = nd.U[par ^ 1] + nd.U_stride * slot + foff[4 * (size_t)c + 1];
+        const size_t tot = (size_t)cnR * cnR;
+        for (size_t idx0 = gtid; idx0 < tot; idx0 += (size_t)4 * GT) {
+            double *dst[4];
+            double v[4], a[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const size_t idx = idx0 + (size_t)k * GT;
+                dst[k] = nullptr;
+                if (idx < tot) {
+                    const int r = (int)(idx % cnR), cc = (int)(idx / cnR);
+                    dst[k] = nd_lu_at(L, Ut, U, nP, nF, nR, umap[r], umap[cc]);
+                    a[k] = cU[idx];
+                }
+            }
+#pragma unroll
+            for (int k = 0; k < 4; ++k) v[k] = dst[k] ? *dst[k] : 0.0;
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+                if (dst[k]) *dst[k] = v[k] + a[k];
+        }
+        csync();
+    }
+    // ---- blocked partial LU of the first nP rows and columns
+    int bad = 0;
+    for (int kb = 0; kb < nP; kb += NB) {
+        const int nb = min(NB, nP - kb), k1 = kb + nb, ntr = nF - k1;
+        for (int idx = tid; idx < NB * NB; idx += T) {
+            const int r = idx / NB, c = idx - r * NB;
+            S0[idx] = (r < nb && c < nb) ? *nd_lu_at(L, Ut, U, nP, nF, nR, kb + r, kb + c) : (r == c ? 1.0 : 0.0);
+        }
+        __syncthreads();
+        if (warp == 0) nd_lu_diag_block<NB>(S0, S, dinv, nb, lane, bad);
+        __syncthreads();
+        // panels, one thread per trailing index rr: row k1+rr of L21 = F21 U11⁻¹ into PL, column k1+rr of U12 = L11⁻¹ F12
+        // into PU; entries up to the next multiple of 32 are zero
+        const int ntr32 = (ntr + 31) & ~31;
+        for (int rr = tid; rr < ntr32; rr += T) {
+            double x[NB];
+            if (rr < ntr) {
+#pragma unroll
+                for (int c = 0; c < NB; ++c) x[c] = c < nb ? L[(size_t)(kb + c) * nF + k1 + rr] : 0.0;
+#pragma unroll
+                for (int c = 0; c < NB; ++c) {
+                    double s0 = x[c], s1 = 0.0;
+#pragma unroll
+                    for (int k = 0; k < c; k += 2) {
+                        s0 = fma(-S[k * NB + c], x[k], s0);
+                        if (k + 1 < c) s1 = fma(-S[(k + 1) * NB + c], x[k + 1], s1);
+                    }
+                    x[c] = (s0 + s1) * dinv[c];
+                    PL[c * PR + rr] = c < nb ? x[c] : 0.0;
+                }
+#pragma unroll
+                for (int c = 0; c < NB; ++c) x[c] = c < nb ? Ut[(size_t)(kb + c) * nF + k1 + rr] : 0.0;
+#pragma unroll
+                for (int c = 0; c < NB; ++c) {
+                    double s0 = x[c], s1 = 0.0;
+#pragma unroll
+                    for (int k = 0; k < c; k += 2) {
+                        s0 = fma(-S[c * NB + k], x[k], s0);
+                        if (k + 1 < c) s1 = fma(-S[c * NB + k + 1], x[k + 1], s1);
+                    }
+                    x[c] = s0 + s1;
+                    PU[c * PR + rr] = c < nb ? x[c] : 0.0;
+                }
+            } else {
+#pragma unroll
+                for (int c = 0; c < NB; ++c) { PL[c * PR + rr] = 0.0; PU[c * PR + rr] = 0.0; }
+            }
+        }
+        __syncthreads();
+        if (CL) csync();        // every CTA has read the block's rows and columns before they are overwritten
+        if (crank == 0)
+            for (int idx = tid; idx < NB * NB; idx += T) {
+                const int r = idx / NB, c = idx - r * NB;
+                if (r < nb && c < nb) {
+                    if (c < r) L[(size_t)(kb + c) * nF + kb + r] = S[idx];
+                    else {
+                        Ut[(size_t)(kb + r) * nF + kb + c] = S[idx];
+                        if (c == r) L[(size_t)(kb + c) * nF + kb + r] = 1.0;
+                    }
+                }
+            }
+        for (int idx = gtid; idx < ntr * nb; idx += GT) {
+            const int c = idx / ntr, rr = idx - c * ntr;
+            const double vl = PL[c * PR + rr], vu = PU[c * PR + rr];
+            L[(size_t)(kb + c) * nF + k1 + rr] = vl;
+            Ut[(size_t)(kb + c) * nF + k1 + rr] = vu;
+            if (!(fabs(vl) <= ND_DMAX) || !(fabs(vu) <= ND_DMAX)) bad = 1;
+        }
+        // trailing update F22 −= PL PUᵀ over all 32×32 warp tiles, 4 rows × 8 columns per thread
+        const int nt = ntr32 >> 5, ntiles = nt * nt;
+        const int li = lane & 7, lj = lane >> 3;
+        for (int wt = crank * nwarps + warp; wt < ntiles; wt += csize * nwarps) {
+            const int ti = wt / nt, tj = wt - ti * nt;
+            const int i0 = 32 * ti + 4 * li, j0 = 32 * tj + 8 * lj;
+            if (i0 >= ntr || j0 >= ntr) continue;
+            double acc[4][8];
+#pragma unroll
+            for (int y = 0; y < 8; ++y)
+#pragma unroll
+                for (int x = 0; x < 4; ++x) {
+                    const int r = i0 + x, cc = j0 + y;
+                    acc[x][y] = (r < ntr && cc < ntr) ? *nd_lu_at(L, Ut, U, nP, nF, nR, k1 + r, k1 + cc) : 0.0;
+                }
+#pragma unroll 4
+            for (int c = 0; c < NB; ++c) {
+                const double *pl = PL + c * PR, *pu = PU + c * PR;
+                const double2 a0 = *reinterpret_cast<const double2 *>(pl + i0);
+                const double2 a1 = *reinterpret_cast<const double2 *>(pl + i0 + 2);
+                const double2 b0 = *reinterpret_cast<const double2 *>(pu + j0);
+                const double2 b1 = *reinterpret_cast<const double2 *>(pu + j0 + 2);
+                const double2 b2 = *reinterpret_cast<const double2 *>(pu + j0 + 4);
+                const double2 b3 = *reinterpret_cast<const double2 *>(pu + j0 + 6);
+                const double pi[4] = {-a0.x, -a0.y, -a1.x, -a1.y};
+                const double pj[8] = {b0.x, b0.y, b1.x, b1.y, b2.x, b2.y, b3.x, b3.y};
+#pragma unroll
+                for (int x = 0; x < 4; ++x)
+#pragma unroll
+                    for (int y = 0; y < 8; ++y) acc[x][y] = fma(pi[x], pj[y], acc[x][y]);
+            }
+#pragma unroll
+            for (int y = 0; y < 8; ++y)
+#pragma unroll
+                for (int x = 0; x < 4; ++x) {
+                    const int r = i0 + x, cc = j0 + y;
+                    if (r < ntr && cc < ntr) *nd_lu_at(L, Ut, U, nP, nF, nR, k1 + r, k1 + cc) = acc[x][y];
+                }
+        }
+        csync();
+    }
+    if (bad) atomicAdd(nd.info + 4 * slot + 1, 1);
+}
+
+// the LU kernels, one per (cluster, block width, panel place) as the Cholesky's; `guard` is unused (no pivot is raised)
+__global__ void __launch_bounds__(512) nd_lu_factor_kernel(NdDev nd, int t0, int par, double, int nFmax) { nd_lu_factor_body<false, ND_NB>(nd, t0, par, nFmax); }
+__global__ void __launch_bounds__(512) nd_lu_factor_cluster_kernel(NdDev nd, int t0, int par, double, int nFmax) { nd_lu_factor_body<true, ND_NB>(nd, t0, par, nFmax); }
+__global__ void __launch_bounds__(512) nd_lu_factor8_kernel(NdDev nd, int t0, int par, double, int nFmax) { nd_lu_factor_body<false, 8>(nd, t0, par, nFmax); }
+__global__ void __launch_bounds__(512) nd_lu_factor8_cluster_kernel(NdDev nd, int t0, int par, double, int nFmax) { nd_lu_factor_body<true, 8>(nd, t0, par, nFmax); }
+__global__ void __launch_bounds__(512) nd_lu_factor_large_kernel(NdDev nd, int t0, int par, double, int nFmax) { nd_lu_factor_body<false, ND_NB, true>(nd, t0, par, nFmax); }
+__global__ void __launch_bounds__(512) nd_lu_factor_large_cluster_kernel(NdDev nd, int t0, int par, double, int nFmax) { nd_lu_factor_body<true, ND_NB, true>(nd, t0, par, nFmax); }
+__global__ void __launch_bounds__(512) nd_lu_factor8_large_kernel(NdDev nd, int t0, int par, double, int nFmax) { nd_lu_factor_body<false, 8, true>(nd, t0, par, nFmax); }
+__global__ void __launch_bounds__(512) nd_lu_factor8_large_cluster_kernel(NdDev nd, int t0, int par, double, int nFmax) { nd_lu_factor_body<true, 8, true>(nd, t0, par, nFmax); }
 
 // dynamic shared memory of the solve kernels (bytes): the front's vector, the ring sums of the backward sweep (both in
 // global memory on the large-front variants), two diagonal blocks (the next one is fetched while the current one is
@@ -1117,6 +1410,7 @@ struct NdLevelPlan {
     int arena_f, arena_s;       // small kernels: arena (doubles)
     bool large_f = false;       // generic factorisation with the panel in global memory (nd_factor_*large*)
     bool large_s = false;       // generic solves with the front vector in global memory (nd_fwd/bwd_large_kernel)
+    bool lu = false;            // LU form (nd_lu_factor_*): two panels, every level on the generic factorisation
 };
 static inline NdLevelPlan nd_level_plan(const NdSymbolic &sym, int s, int mb, double typ_per_pixel, int max_warps_f = 16,
                                        int max_threads_s = 512)
@@ -1166,7 +1460,7 @@ static inline NdLevelPlan nd_level_plan_sized(const NdSymbolic &sym, int s, int 
 }
 
 // shared memory of the generic kernels of a level, as they will be launched
-static inline size_t nd_level_smem_f(const NdLevelPlan &lp) { return nd_factor_smem(lp.nFw, lp.nRc, lp.nb, lp.large_f); }
+static inline size_t nd_level_smem_f(const NdLevelPlan &lp) { return nd_factor_smem(lp.nFw, lp.nRc, lp.nb, lp.large_f, lp.lu); }
 static inline size_t nd_level_smem_s(const NdLevelPlan &lp) { return nd_solve_smem(lp.nFw, lp.large_s); }
 
 // Sends the generic kernels of a level to the large-front variants when their shared memory would exceed `limit` bytes
@@ -1174,9 +1468,17 @@ static inline size_t nd_level_smem_s(const NdLevelPlan &lp) { return nd_solve_sm
 // (half the steps, half the passes over the trailing matrix); a level sent by the hook alone keeps its block width, and
 // so its bits.  false: the level needs the variants for a front beyond `smem_optin` but `allow` is not set — the caller
 // lets a band solver try the shape first, as before the variants existed.
+// A level in the LU form (before nd_level_large): 8-column block steps when the two 16-column panels do not fit in
+// `smem_optin` (the largest front of a 512² image: 1536 unknowns, 393 KB at 16 columns, 203 KB at 8).
+static inline void nd_level_lu(NdLevelPlan &lp, size_t smem_optin)
+{
+    lp.lu = true;
+    if (nd_factor_smem(lp.nFw, lp.nRc, ND_NB, false, true) > smem_optin) lp.nb = 8;
+}
+
 static inline bool nd_level_large(NdLevelPlan &lp, size_t limit, size_t smem_optin, bool allow)
 {
-    const size_t f = nd_factor_smem(lp.nFw, lp.nRc, lp.nb), s = nd_solve_smem(lp.nFw);
+    const size_t f = nd_factor_smem(lp.nFw, lp.nRc, lp.nb, false, lp.lu), s = nd_solve_smem(lp.nFw);
     if (!allow && (f > smem_optin || s > smem_optin)) return false;
     lp.large_f = f > limit;
     lp.large_s = s > limit;
@@ -1189,7 +1491,7 @@ static inline bool nd_level_large(NdLevelPlan &lp, size_t limit, size_t smem_opt
 // vector and the ring sums per front
 static inline size_t nd_level_scratch(const NdLevelPlan &lp, int C)
 {
-    const size_t f = lp.large_f ? (size_t)lp.nfr * C * lp.nb * nd_panel_pitch(lp.nFw) : 0;
+    const size_t f = lp.large_f ? (size_t)lp.nfr * C * (lp.lu ? 2 : 1) * lp.nb * nd_panel_pitch(lp.nFw) : 0;
     const size_t s = lp.large_s ? (size_t)lp.nfr * 2 * nd_even(lp.nFw) : 0;
     return std::max(f, s);
 }

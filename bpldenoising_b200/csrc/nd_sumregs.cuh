@@ -5,13 +5,15 @@
 //
 // with the three difference operators (forward, backward, centred).  For SCALAR α_k the matrix is symmetric positive
 // definite, one unknown per node, and couples nodes at most two pixels apart (G_kᵀ T G_k reaches ±2 rows / columns): the
-// nested-dissection multifrontal Cholesky of the TV learning function takes it with coupling radius W = 2.  (The PATCH
-// variant, :195-262, scales the rows of each term by a different map — not symmetric — and stays on the band LU.)
+// nested-dissection multifrontal Cholesky of the TV learning function takes it with coupling radius W = 2.  The PATCH
+// variant, :195-262, scales the rows of each term by a different map: not symmetric, it takes the LU form of the same
+// fronts (nd_lu_factor_body) on the stencil of nd3_stencil_map_kernel.
 // The per-(pixel, operator) tensors and weights are lu3_classify's, the matrix-free residual is lu3_apply, the functional
 // and the backward-error rule are those of lu3_solve (lu_band.cuh): the band LU remains the second implementation.
 //
-// Kernels: nd3_stencil (the matrix in pixel-stencil form + the right-hand side), nd3_residual (r − M p through the stencils
-// and tensors, independent of the assembled matrix), nd3_axpy, nd3_finish (backward error, functional, sums).
+// Kernels: nd3_stencil / nd3_stencil_map (the matrix in pixel-stencil form + the right-hand side), nd3_residual (r − M p
+// through the stencils and tensors, independent of the assembled matrix), nd3_axpy, nd3_finish (backward error,
+// functional, sums).
 #pragma once
 #include "lu_band.cuh"
 #include "nd_solver.cuh"
@@ -66,9 +68,62 @@ __global__ void __launch_bounds__(256) nd3_stencil_kernel(LuSlots ws, Lu3Params 
     }
 }
 
-// work = r − M p (matrix-free), relres = ‖work‖ / ‖r‖.  One CTA per image.
+// Row v of I + Σ_k diag(α_k) G_kᵀ T_k G_k with the λ-maps α_k (rows scaled by α_k(v): not symmetric), in the LU form's
+// stencil (nd_lu_factor_body: 2·ND3_NH − 1 entries per node) — the values and summation order of lu3_assemble:
+//   [0] A[v, v],  [h] A[v + d_h, v],  [ND3_NH − 1 + h] A[v, v + d_h]
+// Row v gives A[v, v + d_h] of its own node and A[v, v − d_h], the [h] entry of node v − d_h (written only for nodes
+// inside the image, so every entry has one writer); p ← r.  The slot's `ast` must be zero.  grid (slots, chunks)
+constexpr int ND3_NH2 = 2 * ND3_NH - 1;
 template <typename Real>
-__global__ void __launch_bounds__(1024) nd3_residual_kernel(LuSlots ws, Lu3Params pr, double *relres_img, int img0)
+__global__ void __launch_bounds__(256) nd3_stencil_map_kernel(LuSlots ws, Lu3Params pr, const Real *alpha_maps, double *ast_all,
+                                                              size_t ast_stride)
+{
+    const int slot = blockIdx.x;
+    const int n = ws.n, N = ws.N;
+    double *pix = ws.pix + ws.pix_stride * slot;
+    double *ast = ast_all + ast_stride * slot;
+    const int offs[13] = {-2 * n, -n - 1, -n, -n + 1, -2, -1, 0, 1, 2, n - 1, n, n + 1, 2 * n};   // distinct for n ≥ 4
+    const int di[6] = {1, 2, -1, 0, 1, 0}, dj[6] = {0, 0, 1, 1, 1, 2};     // forward offsets of offs[7..12]
+    for (int v = blockIdx.y * blockDim.x + threadIdx.x; v < N; v += gridDim.y * blockDim.x) {
+        const int i = v % n, j = v / n;
+        double acc[13];
+#pragma unroll
+        for (int s = 0; s < 13; ++s) acc[s] = 0.0;
+        acc[6] = 1.0;
+        visit_node(i, j, n, [&](int q, int k, double c1, double c2) {
+            if (k >= ws.nops) return;
+            const double *tk = pix + (size_t)(6 * k) * N;
+            const double a = lu3_alpha<Real>(alpha_maps, pr, N, k, v);
+            const double v1 = c1 * tk[q] + c2 * tk[(size_t)2 * N + q];                  // (c1 c2)·T
+            const double v2 = c1 * tk[(size_t)N + q] + c2 * tk[(size_t)3 * N + q];
+            visit_stencil(k, q % n, q / n, n, [&](int node, double e1, double e2) {
+                const double val = a * (v1 * e1 + v2 * e2);
+                const int d = node - v;
+#pragma unroll
+                for (int s = 0; s < 13; ++s)
+                    if (offs[s] == d) { acc[s] += val; break; }
+            });
+        });
+        double *row = ast + (size_t)v * ND3_NH2;
+        row[0] = acc[6];
+#pragma unroll
+        for (int s = 0; s < 6; ++s) {
+            const int h = nd3_h(di[s], dj[s]);
+            row[ND3_NH - 1 + h] = acc[7 + s];                       // A[v, v + d_h]
+            const int ii = i - di[s], jj = j - dj[s];               // A[v, v − d_h] = A[w + d_h, w], w = v − d_h
+            if (ii >= 0 && ii < n && jj >= 0 && jj < n) ast[(size_t)(ii + n * jj) * ND3_NH2 + h] = acc[5 - s];
+        }
+        pix[(size_t)LU_PL_P * N + v] = pix[(size_t)LU_PL_R * N + v];
+    }
+}
+
+// work = r − M p (matrix-free; the λ-maps when given), relres = ‖work‖ / ‖r‖.  One CTA per image.
+// rstate (2 doubles per slot, or nullptr): the stop of lu3_solve's refinement at step `it` (0: after the first solve) —
+// after pr.refine steps, at rounding level, or when a step no longer gains a factor 4, rstate[1] is set and nd3_axpy
+// leaves p alone from then on (the residual of the unchanged p is formed again, with the same bits).
+template <typename Real>
+__global__ void __launch_bounds__(1024) nd3_residual_kernel(LuSlots ws, Lu3Params pr, double *relres_img, int img0,
+                                                            const Real *alpha_maps = nullptr, double *rstate = nullptr, int it = 0)
 {
     __shared__ double red[40];
     const int slot = blockIdx.x, tid = threadIdx.x;
@@ -78,20 +133,32 @@ __global__ void __launch_bounds__(1024) nd3_residual_kernel(LuSlots ws, Lu3Param
     double *work = pix + (size_t)LU_PL_WORK * N;
     double bn2 = 0.0, rn2 = 0.0;
     for (int v = tid; v < N; v += blockDim.x) {
-        const double res = r[v] - lu3_apply<Real>(pix, n, N, ws.nops, nullptr, pr, p, v);
+        const double res = r[v] - lu3_apply<Real>(pix, n, N, ws.nops, alpha_maps, pr, p, v);
         work[v] = res;
         rn2 = fma(res, res, rn2);
         bn2 = fma(r[v], r[v], bn2);
     }
     rn2 = lu_block_sum(rn2, red);
     bn2 = lu_block_sum(bn2, red);
-    if (tid == 0) relres_img[img0 + slot] = bn2 > 0.0 ? sqrt(rn2 / bn2) : 0.0;
+    if (tid == 0) {
+        const double rel = bn2 > 0.0 ? sqrt(rn2 / bn2) : 0.0;
+        relres_img[img0 + slot] = rel;
+        if (rstate) {
+            double *rs = rstate + 2 * slot;       // [0] residual of the last step taken, [1] ≠ 0: stopped
+            if (it == 0) { rs[0] = 1e300; rs[1] = 0.0; }
+            if (rs[1] == 0.0) {
+                if (it >= pr.refine || rel <= 1e-14 || !(rel <= 0.25 * rs[0])) rs[1] = 1.0;
+                else rs[0] = rel;
+            }
+        }
+    }
 }
 
-// p += work.  grid (slots, chunks)
-__global__ void __launch_bounds__(256) nd3_axpy_kernel(LuSlots ws)
+// p += work (not once the slot's refinement stopped: rstate as nd3_residual_kernel).  grid (slots, chunks)
+__global__ void __launch_bounds__(256) nd3_axpy_kernel(LuSlots ws, const double *rstate = nullptr)
 {
     const int slot = blockIdx.x, N = ws.N;
+    if (rstate && rstate[2 * slot + 1] != 0.0) return;
     double *pix = ws.pix + ws.pix_stride * slot;
     double *p = pix + (size_t)LU_PL_P * N;
     const double *work = pix + (size_t)LU_PL_WORK * N;
@@ -101,9 +168,11 @@ __global__ void __launch_bounds__(256) nd3_axpy_kernel(LuSlots ws)
 // Normwise backward error ‖r − Mp‖ / (‖M‖‖p‖ + ‖r‖) with the bound ‖M‖ ≤ 1 + 18·γ·max α (as lu3_solve) → relres_img; a
 // factorisation that broke down or an error above `tol` poisons the result with NaN (→ BPLTV_ERR_NUMERIC).
 // g_k = Σ_v p_v (G_kᵀ w_k)_v per operator (:166), summed per patch of the lm×ln grid (1×1 for the scalar parameter).
-// `work` must hold the residual of the final p.  One CTA per image.
+// With the λ-maps (:195-262), max α runs over the maps and relres_img keeps the relative residual ‖r − Mp‖/‖r‖ of
+// nd3_residual_kernel, as lu3_solve reports it.  `work` must hold the residual of the final p.  One CTA per image.
+template <typename Real = double>
 __global__ void __launch_bounds__(1024) nd3_finish_kernel(LuSlots ws, Lu3Params pr, const int *nd_info, double tol, double *out_img,
-                                                         double *relres_img, int img0)
+                                                         double *relres_img, int img0, const Real *alpha_maps = nullptr)
 {
     __shared__ double red[40];
     const int slot = blockIdx.x, tid = threadIdx.x;
@@ -121,7 +190,13 @@ __global__ void __launch_bounds__(1024) nd3_finish_kernel(LuSlots ws, Lu3Params 
     bn2 = lu_block_sum(bn2, red);
     rn2 = lu_block_sum(rn2, red);
     double amax = 0.0;
-    for (int k = 0; k < ws.nops; ++k) amax = fmax(amax, pr.alpha[k]);
+    if (alpha_maps) {
+        for (int v = tid; v < N; v += blockDim.x)
+            for (int k = 0; k < ws.nops; ++k) amax = fmax(amax, lu3_alpha<Real>(alpha_maps, pr, N, k, v));
+        amax = lu_block_max(amax, red);
+    } else {
+        for (int k = 0; k < ws.nops; ++k) amax = fmax(amax, pr.alpha[k]);
+    }
     const double berr = sqrt(rn2) / ((1.0 + 18.0 * pr.gamma * amax) * sqrt(pn2) + sqrt(bn2) + 1e-300);
     const bool failed = nd_info[4 * slot + 1] != 0 || !(berr <= tol);
     const int ng = pr.lm * pr.ln;
@@ -148,7 +223,7 @@ __global__ void __launch_bounds__(1024) nd3_finish_kernel(LuSlots ws, Lu3Params 
         }
         __syncthreads();
     }
-    if (tid == 0) relres_img[img0 + slot] = berr;
+    if (tid == 0 && !alpha_maps) relres_img[img0 + slot] = berr;
 }
 
 

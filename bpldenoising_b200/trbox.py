@@ -278,7 +278,8 @@ def scalar_bilevel_sumregs_learn(data, ctx=None, **kwargs) -> LearnResult:
 def patch_bilevel_sumregs_learn(data, ctx=None, **kwargs) -> LearnResult:
     """patch_bilevel_sumregs_learn (BPLDenoising.jl:464-481) without IO/visualisation.  Once the trust
     region shrinks below Δt = 1e-3 the learning function switches to the patch variant of
-    sumregs_gradient_reg (SumRegsLearningFunction.jl:195-262), which libbpltv solves with its band LU."""
+    sumregs_gradient_reg (SumRegsLearningFunction.jl:195-262), which libbpltv solves with its band LU up to 430²
+    and with the LU of its nested-dissection fronts beyond."""
     from .learning import sumregs_learning_function
 
     prm = dict(PATCH_SUMREGS_BILEVEL_PARAMS); prm.update(kwargs)

@@ -94,7 +94,9 @@ typedef struct bpltv_eval_opts {
                             (one SM per image), kept as a second implementation.  Sum of
                             regularisers: the symmetric variants (sumregs_gradient scalar
                             and patch, scalar sumregs_gradient_reg) follow this switch; the
-                            row-scaled patch sumregs_gradient_reg is always the band LU   */
+                            row-scaled patch sumregs_gradient_reg takes the band LU, and
+                            above 430² (where the band LU refuses) the LU of the
+                            nested-dissection fronts; solver 1 keeps it on the band LU   */
     int force_branch;    /* 0: by Δ (reference); 1: gradient; 2: gradient_reg;
                             3: cost only (grad_out left zero; λ-sweeps, validation)  */
     int reserved0;
@@ -114,11 +116,12 @@ typedef struct bpltv_stats {
                                     entry points).  Nested dissection (solver 0/2): the normwise
                                     backward error that solver_tol bounds (TV, scalar
                                     sumregs_gradient_reg) or the relative residual |r|/|b| of the
-                                    multiplier system (sumregs_gradient).  Banded solvers (solver 1,
-                                    patch sumregs_gradient_reg): the relative residual |r|/|b| after the
-                                    last refinement step — informational (with entries up to
-                                    alpha*gamma it is not a backward error); the band LU applies its
-                                    own backward-error test and poisons the gradient with NaN      */
+                                    multiplier system (sumregs_gradient).  Banded solvers (solver 1) and
+                                    patch sumregs_gradient_reg (band LU or the fronts' LU): the relative
+                                    residual |r|/|b| after the last refinement step — informational
+                                    (with entries up to alpha*gamma it is not a backward error); both
+                                    LUs apply their own backward-error test and poison the gradient
+                                    with NaN                                                         */
     int pdps_kernel_used;        /* enum bpltv_pdps_kernel actually dispatched */
     int n_devices;
     int tblock_depth;            /* PDPS iterations per HBM pass of that kernel (1 unless TBLOCK) */
@@ -198,10 +201,10 @@ int bpltv_sumregs_denoise(bpltv_ctx *ctx, const double *noisy, int M, int N, int
  * : sumregs_gradient_reg (:112-167), summed over images (:87-110, :169-193).  grad_out has the shape
  * of x: 3 (lm = ln = 1) or lm×ln×3 entries.  The patch variant of sumregs_gradient_reg (:195-262),
  * whose system is row-scaled by a different λ-map per operator and therefore not symmetric, is
- * solved by a banded LU in node space (γ = opts->gamma_patch) and is limited to M = N ≤ 430 (it
- * would need an unsymmetric multifrontal LU).  The symmetric variants take any square size: where
- * the fronts of the nested-dissection solver outgrow shared memory and the band solvers refuse
- * the size too, its large-front kernels (panel and front vector in global memory) take over; an
+ * solved by a banded LU in node space (γ = opts->gamma_patch) up to M = N ≤ 430 and by an LU of the
+ * nested-dissection fronts beyond.  Every variant takes any square size: where the fronts of the
+ * nested-dissection solver outgrow shared memory and the band solvers refuse the size too, its
+ * large-front kernels (panels and front vector in global memory) take over; an
  * image whose workspace does not fit in device memory returns BPLTV_ERR_ALLOC, and
  * bpltv_last_error names the gigabytes one image needs.  opts == NULL → the
  * sum-of-regularisers defaults.                                                              */
